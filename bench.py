@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the RQAE residual-quantization hot path (forward = encode + reconstruction).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--tokens T]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--tokens T] [--dump-outputs DIR]
 
 One "step" = one pass of RQAE.forward over T synthetic N(0,1) activation tokens per GPU at Gemma-2-2B
 width (d=2304, nq=1024, K=625, random init from torch.manual_seed(0)): BASELINE.json configs[1].
@@ -13,6 +13,10 @@ rank processes its own T tokens (weak scaling), no collective on the data path.
 `--impl reference` times the reference's CPU implementation of the same path on the host cores: the
 unmodified /root/reference module when it exists (build container), else the op-for-op torch port in
 oracle/rqae_oracle.py (the GPU box has no /root/reference).
+
+`--dump-outputs DIR` writes what RQAE.forward returned in the last timed step (rank 0's tokens) as
+DIR/quantized_out.npy (float32) and DIR/indices.npy (float64, exact for the int64 codes), at the same seeded sample
+of token rows on every run, so that two builds given the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -31,6 +35,7 @@ FLOP_PER_TOKEN_FWD = NQ * 46472          # SURVEY 8d: 2*4*D in-proj + 2*4*K cos 
 HBM_BYTES_PER_TOKEN_FWD = 4 * D + 8 * NQ + 4 * D   # x in, int64 codes out, fp32 reconstruction out
 METRIC = "rq_forward_encode_decode_tokens_per_sec"
 UNIT = "tokens/s"
+DUMP_ROWS = 3072    # token rows of --dump-outputs: 3072 x (2304 x 4 B + 1024 x 8 B) = 53.5 MB, within 64 MB
 
 
 def parse():
@@ -49,7 +54,15 @@ def parse():
     ap.add_argument("--no-parity", action="store_true", help="skip the 4096-token KAT parity block")
     ap.add_argument("--tokens-9b", type=int, default=1 << 20, help="tokens per GPU of the configs[3] extra")
     ap.add_argument("--tokens-mining", type=int, default=1 << 21, help="tokens per GPU of the configs[4] extra")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (a fixed sample of %d token rows) as DIR/<name>.npy"
+                         % DUMP_ROWS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -634,6 +647,17 @@ def config4_mining_extra(torch, dist, model, x, dev, rank, world, tokens, n_feat
     return res
 
 
+def dump_outputs(torch, out_dir, q, codes):
+    """quantized_out (1, T, D) and indices (1, T, nq) of RQAE.forward at DUMP_ROWS token rows (all of them when
+    T is smaller), ascending; the rows are drawn from a fixed seed and depend on T alone."""
+    import numpy as np
+    rows = torch.randperm(codes.shape[1], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    rows = rows.to(codes.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "quantized_out.npy"), q[0, rows].cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "indices.npy"), codes[0, rows].cpu().numpy().astype(np.float64))
+
+
 def run_b200(args, rank, local_rank, world):
     import torch
     import torch.distributed as dist
@@ -703,6 +727,8 @@ def run_b200(args, rank, local_rank, world):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     checksum = int(codes.sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, q, codes)
     del q, codes
     ms_step = ms / args.steps
     value = world * T / (ms_step * 1e-3)
