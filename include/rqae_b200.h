@@ -191,8 +191,8 @@ int rqae_intensity_again_f16(const float* cb_norm, int K, int64_t n_tokens, cons
  * Rows of 16 384 .. 262 144 values go through the sample-bracketed single-pass kernel (rq_mine3.cuh); a row whose
  * brackets miss, and every other row length, through the three-pass kernel (rq_mine.cuh) -- same result, same order.
  * The call takes a few bytes per row from a stream-ordered pool of the library (cudaMallocFromPoolAsync on `stream`) for the
- * fallback list.  Environment, read per call: RQAE_MINE_V2=1 three-pass kernel only, RQAE_MINE_V1=1 the first version
- * (both for A/B timing), RQAE_M3_PROF=1 per-step clocks on stderr (synchronises). */
+ * fallback list.  Environment, read per call: RQAE_MINE_V2=1 runs the three-pass kernel for every row (A/B timing of
+ * the two kernels; the only selection switch). */
 int rqae_select_top_middle_bottom_f16(const void* vals, int64_t rows, int64_t row_stride, int64_t n, int top_k,
                                       int32_t* idx_out, void* val_out, void* stream);
 
@@ -282,10 +282,6 @@ int rqae_search_tc_maxima_f16(const void* store_tc, int64_t n_seq, int seq_len, 
 int rqae_search_rows_f16(const void* table, int K, const void* codes, int code_dtype, int64_t code_stride, int64_t n_seq,
                          int seq_len, const int32_t* sel, int n_query, int n_sel, const int32_t* layers_host,
                          int first_range, int n_cuts, void* rows_out, void* stream);
-
-/* Measurement helper: per-CTA clock counters (16 x uint64 per CTA, meaning in rq_intensity.cuh) written by the last
- * rqae_intensity_f16 launch that ran with the environment variable RQAE_INT_DBG having bit 1024 set; synchronises. */
-int rqae_intensity_profile(uint64_t* out_host, int n_ctas);
 
 /* Number of kernels this library has launched on this thread since the last reset
  * (bench.py reports it as gpu_launches). */

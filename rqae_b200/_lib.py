@@ -17,7 +17,7 @@ LIB_PATH = os.environ.get("RQAE_B200_LIB") or os.path.join(_HERE, "librqae_b200.
 SYMBOLS = [
     "rqae_version", "rqae_strerror", "rqae_last_cuda_error", "rqae_packed_bytes", "rqae_pack_weights",
     "rqae_forward_f32", "rqae_forward_variant", "rqae_hook_rmsnorm", "rqae_decode_f32", "rqae_forward_host_f32", "rqae_forward_host_config", "rqae_forward_host_mode", "rqae_widen_codes_host", "rqae_forward_host_release",
-    "rqae_fp32_peak_probe", "rqae_intensity_profile", "rqae_intensity_again_f16", "rqae_search_tc_store_bytes", "rqae_search_tc_pack_store",
+    "rqae_fp32_peak_probe", "rqae_intensity_again_f16", "rqae_search_tc_store_bytes", "rqae_search_tc_pack_store",
     "rqae_search_tc_workspace_bytes", "rqae_search_tc_maxima_f16", "rqae_search_rows_f16", "rqae_search_qrows_bytes",
     "rqae_search_build_qrows_f16",
     "rqae_launch_count", "rqae_intensity_workspace_bytes", "rqae_intensity_f16",
@@ -72,8 +72,6 @@ def load() -> ctypes.CDLL:
     lib.rqae_forward_host_release.argtypes = []
     lib.rqae_fp32_peak_probe.restype = i
     lib.rqae_fp32_peak_probe.argtypes = [i, i, c.POINTER(c.c_double), vp, vp]
-    lib.rqae_intensity_profile.restype = i
-    lib.rqae_intensity_profile.argtypes = [vp, i]
     lib.rqae_intensity_workspace_bytes.restype = sz
     lib.rqae_intensity_workspace_bytes.argtypes = [vp, i, i, i64]
     lib.rqae_intensity_f16.restype = i

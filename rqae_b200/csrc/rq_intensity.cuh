@@ -99,8 +99,7 @@ struct IntParams {
   __half* s_max;          // [n_cuts][128][s_stride]: max over the positions of every sequence
   long long s_stride;     // >= 2 * n_units, even
   int s_len, L8;          // positions per sequence (<= 128), 8-layer blocks per token
-  int stagger, stagger_groups;   // clocks between the start groups of CTAs (0: all together), number of groups
-  int dbg;   // timing experiments only (RQAE_INT_DBG): 1 no output stores, 2 no table look-ups, 4 no pause at cuts, 8 no MMA, 16 no epilogue work, 64 no feature-operand copies, 128 no code loads, 256 no proxy fence in the builders, 512 no L2 prefetch of code rows, 1024 per-role clock counters (g_int_prof)
+  int stagger;            // clocks between the start groups of CTAs (0: all start together)
 };
 
 struct IntSmem {
@@ -240,15 +239,6 @@ __device__ __forceinline__ void mbar_wait_spin(uint64_t* bar, uint32_t parity) {
   } while (!ok);
 }
 
-// Per-CTA clock counters of the last launch run with dbg bit 1024 (measurement only; read by rqae_intensity_profile):
-// [0] issuer: waiting for a token stage, [1] for a feature tile, [2] for an accumulator, [3] issuer total,
-// [4] builder: waiting for a free stage, [5] look-ups and stores, [6] builder total,
-// [7] epilogue warp: waiting for a cut, [8] holding the accumulator, [9] waiting for its stores to read, [10] epilogue total,
-// [11] feature-tile producer: waiting for a free stage, [12] producer total,
-// [13] epilogue: cut signalled -> first stores issued (includes [8]), [14] roundings of the kept half, [15] first store-read wait + second staging + stores.
-constexpr int IT_PROF_SLOTS = 16;
-__device__ unsigned long long g_int_prof[256 * IT_PROF_SLOTS];
-
 // EPI = 0: feature intensities (fp16 out[f][cut][t] with the reference's roundings).
 // EPI = 1: tensor-core decode -- "features" are the D output dimensions, U holds W_out, one cut at the last layer,
 //          out is q_out[t][d] fp32 (+ the summed out-projection biases); opt-in, not bit-exact (rq_decode.cuh is).
@@ -301,15 +291,13 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
 
   const int n_pairs = (p.F_tiles + 1) / 2;
   const long long n_units = p.n_tok_tiles * n_pairs;
-  const bool prof = (p.dbg & 1024) != 0 && blockIdx.x < 256;
-  unsigned long long* const pr_out = g_int_prof + (size_t)(blockIdx.x & 255) * IT_PROF_SLOTS;
-  auto tick = [&]() -> long long { return prof ? clock64() : 0ll; };
   if (p.stagger > 0) {
     // De-phase the CTAs: the first ten cuts of scripts/3's list fall into the first ten K-blocks of a unit, so every
     // unit begins with a burst of output (1.3 MB per SM) and, started together, all SMs burst together and wait on
     // HBM writes.  Four start groups a fraction of a unit apart spread the bursts (measured: 1.73 -> 1.63 ms).
+    constexpr int IT_STAGGER_GROUPS = 4;
     const long long t0 = clock64();
-    const long long d = (long long)(blockIdx.x % p.stagger_groups) * p.stagger;
+    const long long d = (long long)(blockIdx.x % IT_STAGGER_GROUPS) * p.stagger;
     while (clock64() - t0 < d) {
     }
     __syncthreads();
@@ -324,28 +312,19 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
     // ======================= U producer =======================
     if (lane == 0) {
       uint32_t s = 0, par = 1;   // a fresh barrier passes a wait on parity 1
-      long long w_e = 0;
-      const long long t_begin = tick();
       for (long long u = blockIdx.x; u < n_units; u += gridDim.x) {
         const int pr = (int)(u % n_pairs);
         const int nft = min(2, p.F_tiles - 2 * pr);
         for (int kb = 0; kb < p.NKB; kb++) {
           for (int ft = 0; ft < nft; ft++) {
-            const long long t0 = tick();
             mbar_wait_spin(&u_empty[s], par);
-            w_e += tick() - t0;
-            if (p.dbg & 64) {   // timing experiment: no feature-operand traffic
-              mbar_arrive(&u_full[s]);
-            } else {
-              mbar_arrive_expect_tx(&u_full[s], IT_U_TILE);
-              tma_bulk_g2s(uring + s * IT_U_TILE, p.u_tiles + ((size_t)(2 * pr + ft) * p.NKB + kb) * (size_t)IT_U_TILE, IT_U_TILE,
-                           &u_full[s]);
-            }
+            mbar_arrive_expect_tx(&u_full[s], IT_U_TILE);
+            tma_bulk_g2s(uring + s * IT_U_TILE, p.u_tiles + ((size_t)(2 * pr + ft) * p.NKB + kb) * (size_t)IT_U_TILE, IT_U_TILE,
+                         &u_full[s]);
             if (++s == USTAGES) { s = 0; par ^= 1; }
           }
         }
       }
-      if (prof) { pr_out[11] = (unsigned long long)w_e; pr_out[12] = (unsigned long long)(tick() - t_begin); }
     }
     __syncwarp();
   } else if (warp == 1) {
@@ -359,41 +338,30 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
       uint32_t vs = 0, vpar = 0, us = 0, upar = 0;
       uint32_t free_par0 = 0, free_par1 = 0;
       bool pend0 = false, pend1 = false;   // accumulator a was handed to its epilogue warps and not yet taken back
-      const bool no_mma = (p.dbg & 8) != 0, no_pause = (p.dbg & 4) != 0;
-      long long w_v = 0, w_u = 0, w_f = 0;
-      const long long t_begin = tick();
       for (long long u = blockIdx.x; u < n_units; u += gridDim.x) {
         const int pr = (int)(u % n_pairs);
         const int nft = min(2, p.F_tiles - 2 * pr);
         for (int kb = 0; kb < p.NKB; kb++) {
           const bool is_cut = sched[kb].cut >= 0;
-          long long t0 = tick();
           mbar_wait_spin(&v_full[vs], vpar);
-          w_v += tick() - t0;
           const uint64_t bd = umma_desc_sw128(vring + vs * IT_V_BYTES);
 #pragma unroll
           for (int ft = 0; ft < 2; ft++) {
             if (ft >= nft) break;
-            t0 = tick();
             mbar_wait_spin(&u_full[us], upar);
-            w_u += tick() - t0;
             bool& pend = ft ? pend1 : pend0;
             uint32_t& free_par = ft ? free_par1 : free_par0;
             if (pend) {   // the epilogue of the previous cut (or of the previous unit's last cut) still owns this accumulator
-              t0 = tick();
-              if (!no_pause) mbar_wait_spin(&acc_free[ft], free_par);
-              w_f += tick() - t0;
+              mbar_wait_spin(&acc_free[ft], free_par);
               free_par ^= 1;
               pend = false;
             }
             tc_fence_after();
             const uint64_t ad = umma_desc_sw128(uring + us * IT_U_TILE);
             if (elect_one()) {
-              if (!no_mma) {
 #pragma unroll
-                for (int k = 0; k < 4; k++)   // 16 k values = 32 bytes inside the swizzle row: start address += 2 (x16 B)
-                  umma_f16(tmem_base + ft * IT_TOK, ad + 2 * k, bd + 2 * k, idesc, (kb | k) != 0);
-              }
+              for (int k = 0; k < 4; k++)   // 16 k values = 32 bytes inside the swizzle row: start address += 2 (x16 B)
+                umma_f16(tmem_base + ft * IT_TOK, ad + 2 * k, bd + 2 * k, idesc, (kb | k) != 0);
               tc_commit(&u_empty[us]);
               if (is_cut) tc_commit(&acc_full[ft]);   // the running prefix goes to its epilogue warps; the other accumulator carries on
             }
@@ -405,10 +373,6 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
           __syncwarp();
           if (++vs == IT_VSTAGES) { vs = 0; vpar ^= 1; }
         }
-      }
-      if (prof && lane == 0) {
-        pr_out[0] = (unsigned long long)w_v; pr_out[1] = (unsigned long long)w_u; pr_out[2] = (unsigned long long)w_f;
-        pr_out[3] = (unsigned long long)(tick() - t_begin);
       }
     }
   }   // warps 2-3: spare warps of the control warpgroup
@@ -479,8 +443,6 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
     const uint32_t sw = (uint32_t)(b & 7);
     const uint32_t csh = (uint32_t)(b >> 7) * 16u;   // the code word holds token (b & 127) in its low and token (b & 127) + 128 in its high half
     uint32_t s = 0, par = 1;
-    long long bw_e = 0, bw_b = 0;
-    const long long bt_begin = tick();
     // The codes of a K-block are 16 coalesced 128-byte warp loads.  They are requested TWO K-blocks ahead into
     // registers, and the K-block IT_PF steps ahead is pulled into L2 with one bulk prefetch: the code rows stream
     // from HBM and their latency must stay off the V hand-over path.
@@ -488,7 +450,7 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
     auto next = [&](Pos& q) { if (++q.kb == p.NKB) { q.kb = 0; q.u += gridDim.x; q.tile = q.u / n_pairs; } };
     auto fetch = [&](uint32_t (&c)[IT_LPB], const Pos& q) {
       const uint32_t padw = (uint32_t)p.K | ((uint32_t)p.K << 16);
-      if (q.u < n_units && !(p.dbg & 128)) {
+      if (q.u < n_units) {
         const int l0 = sched[q.kb].l0, n = sched[q.kb].n;
         const uint32_t* src = p.codes_p + ((size_t)q.tile * p.L + l0) * 128 + (b & 127);
 #pragma unroll
@@ -496,7 +458,7 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
       }
     };
     auto l2_prefetch = [&](const Pos& q) {
-      if (b == 0 && q.u < n_units && !(p.dbg & 512)) {
+      if (b == 0 && q.u < n_units) {
         const int l0 = sched[q.kb].l0, n = sched[q.kb].n;
         const uint32_t* src = p.codes_p + ((size_t)q.tile * p.L + l0) * 128;
         asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(n * 512) : "memory");
@@ -511,12 +473,8 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
       next(fut);
       l2_prefetch(pf);
       next(pf);
-      const long long t0 = tick();
       mbar_wait_spin(&v_empty[s], par);
-      const long long t1 = tick();
-      bw_e += t1 - t0;
       const uint32_t vb = vring + s * IT_V_BYTES;
-      if (!(p.dbg & 2))
 #pragma unroll
       for (int cc = 0; cc < 8; cc++) {
         uint32_t x0, x1, x2, x3;
@@ -526,8 +484,7 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
                      "r"(x1), "r"(x2), "r"(x3)
                      : "memory");
       }
-      if (!(p.dbg & 256)) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the MMA
-      bw_b += tick() - t1;
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the MMA
       mbar_arrive(&v_full[s]);   // (one poller and one arrival per warp instead of all threads was measured: slower, the __syncwarps sit on the hand-over path)
       if (++s == IT_VSTAGES) { s = 0; par ^= 1; }
     };
@@ -543,9 +500,6 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
       if (cur.u >= n_units) break;
       step(cB, cur, fut, pf);
       next(cur);
-    }
-    if (prof && b == 0) {
-      pr_out[4] = (unsigned long long)bw_e; pr_out[5] = (unsigned long long)bw_b; pr_out[6] = (unsigned long long)(tick() - bt_begin);
     }
     }   // EPI != 2
   } else {
@@ -566,8 +520,6 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
     };
     const uint64_t pol = l2_policy_evict_first();   // the intensities are a stream: keep the U tiles and code rows in L2
     uint32_t full_par = 0;
-    long long ew_f = 0, ew_h = 0, ew_r = 0, ew_a = 0, ew_b = 0, ew_c = 0;
-    const long long et_begin = tick();
     for (long long u = blockIdx.x; u < n_units; u += gridDim.x) {
       const int pr = (int)(u % n_pairs);
       const long long tok0 = (u / n_pairs) * IT_TOK;
@@ -576,21 +528,14 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
       for (int kb = 0; kb < p.NKB; kb++) {
         const int cut = sched[kb].cut;
         if (cut < 0) continue;
-        const long long te0 = tick();
         mbar_wait(my_full, full_par);   // idle most of the time: suspended wait, no polling traffic next to the builders
-        const long long te1 = tick();
-        ew_f += te1 - te0;
         full_par ^= 1;
         tc_fence_after();
-        if (p.dbg & 16) {
-          if (lane == 0) mbar_arrive(my_free);
-          continue;
-        }
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * IT_TOK;
         if (EPI == 2) {
           // example search: lane = query position, columns = the positions of two sequences; out = max over positions
           float m0 = -INFINITY, m1 = -INFINITY;
-#pragma unroll
+#pragma unroll 2   // fully unrolled, ptxas keeps more TMEM loads in flight than the registers hold and spills
           for (int ch = 0; ch < IT_TOK / 32; ch++) {
             uint32_t v[32];
             tmem_ld32(taddr + ch * 32, v);
@@ -625,7 +570,7 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
               if (lane == 0) mbar_arrive(my_free);
             }
             float* o = p.q_out + (size_t)(tok0 + ch * 32) * p.D + d;
-            if (d < p.D && !(p.dbg & 1)) {
+            if (d < p.D) {
 #pragma unroll
               for (int j = 0; j < 32; j++)
                 if (tok0 + ch * 32 + j < p.T) __stcs(o + (size_t)j * p.D, __uint_as_float(v[j]) + bsum);
@@ -635,7 +580,7 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
         }
         const float inv = wcum_s[p.n_cuts + cut];
         const int frow0 = (2 * pr + acc) * IT_FT + q * 32;   // the warp's 32 feature rows; rows >= F are clipped by the tensor map
-        const bool do_store = lane == 0 && !(p.dbg & 1);
+        const bool do_store = lane == 0;
         // (1) tokens 0..127 of the row: only the reference's FIRST rounding (prefix -> fp16), kept packed in registers;
         // (2) tokens 128..255: finished and staged (the boxes have been read by the previous cut's stores: that wait
         // sits at the bottom of this loop, not inside the hold).
@@ -648,7 +593,7 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
 #pragma unroll
           for (int j = 0; j < 16; j++) keep[ch * 16 + j] = pack_h2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1]));
         }
-#pragma unroll
+#pragma unroll 2   // fully unrolled, ptxas keeps more TMEM loads in flight than the registers hold and spills the kept half
         for (int ch = 4; ch < 8; ch++) {
           uint32_t v[32];
           tmem_ld32(taddr + ch * 32, v);
@@ -657,7 +602,6 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(my_free);
-            ew_h += tick() - te1;
           }
 #pragma unroll
           for (int g = 0; g < 4; g++)   // all roundings at once: every trip through shared memory competes with the operand traffic
@@ -675,16 +619,11 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
           tma_store_box(&out_map, wstg + IT_STG_BOX, (int)tok0 + 192, cut, frow0, pol);
         }
         if (lane == 0) bulk_commit();
-        const long long teA = tick();
-        ew_a += teA - te1;   // includes the hold
         // (4) the kept half: remaining roundings in registers while the first stores drain, then the same boxes again
 #pragma unroll
         for (int j = 0; j < 64; j++) keep[j] = finish_packed(keep[j], inv);
-        const long long te3 = tick();
-        ew_b += te3 - teA;
         if (lane == 0) bulk_wait_read_all();
         __syncwarp();
-        ew_r += tick() - te3;
 #pragma unroll
         for (int j = 0; j < 16; j++)
           asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg_addr(j)), "r"(keep[4 * j]), "r"(keep[4 * j + 1]),
@@ -698,20 +637,12 @@ __global__ void __launch_bounds__(IT_THREADS, 1) rq_intensity_kernel(const IntPa
         }
         if (lane == 0) bulk_commit();
         // the boxes must have been read before the next cut's prefix is staged: wait here, not while holding TMEM
-        const long long te4 = tick();
-        ew_c += te4 - te3;   // includes the first store-read wait
         if (lane == 0) bulk_wait_read_all();
         __syncwarp();
-        ew_r += tick() - te4;
       }
     }
     if (lane == 0) bulk_wait_all();   // the boxes are read, and the rows written, before the CTA retires
     __syncwarp();
-    if (prof && warp == 12 && lane == 0) {
-      pr_out[7] = (unsigned long long)ew_f; pr_out[8] = (unsigned long long)ew_h; pr_out[9] = (unsigned long long)ew_r;
-      pr_out[10] = (unsigned long long)(tick() - et_begin);
-      pr_out[13] = (unsigned long long)ew_a; pr_out[14] = (unsigned long long)ew_b; pr_out[15] = (unsigned long long)ew_c;
-    }
   }
 
   // ---- teardown ----

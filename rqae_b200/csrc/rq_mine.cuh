@@ -1,15 +1,33 @@
-// Top / middle / bottom-k selection over rows of fp16 intensities (sm_100a).
+// Top / middle / bottom-k selection over rows of fp16 intensities (sm_100a): rq_mine2_kernel, the exact three-pass
+// radix select.
 //
 // Replaces the per-(feature, layer) `torch.argsort(layer_activations, descending=True)` over the whole
 // dataset followed by three slices (scripts/3_make_rqae_features.py:116-128, reference harish-kamath/rqae):
 //     top    = sorted[:k]      middle = sorted[n//2 - k//2 : n//2 + k//2]      bottom = sorted[-k:]
-// with an exact radix select: fp16 has 65 536 values, so two histogram passes (the high 11 bits, then the
-// low 5 bits inside the four bins that hold a window boundary) locate the value at each boundary rank, and
-// a third pass collects the window members.  The total order is (value descending, index ascending);
-// torch's argsort is unstable, so the reference leaves the order among equal values unspecified -- here it
-// is deterministic.  One CTA of 1024 threads per row; the row (4 MB at 2 Mi tokens) stays in L2 between
-// the passes, so HBM sees it once.  Warp w owns the contiguous slice [w, w+1) * ceil(n/32) of the row, which
-// makes "index ascending" among ties a warp-local prefix count plus a per-warp base.
+// fp16 has 65 536 values, so two histogram passes over 8-bit digits locate the value at each window boundary
+// rank, and a third pass collects the window members:
+//   pass 1  histogram of the high key byte (raw bit pattern; bins are visited in descending-value order later)
+//   pass 2  histogram of the low byte inside the bin that holds the median window (lane-private counters, below);
+//           the bins that hold the top / bottom boundaries are tails with few members and use per-warp atomics
+//   pass 3  collects the members of the three windows
+// The total order is (value descending, index ascending; +0 before -0); torch's argsort is unstable, so the
+// reference leaves the order among equal values unspecified -- here it is deterministic.  Warp w owns the
+// contiguous slice [w, w+1) * ceil(n / M2_WARPS) of the row, which makes "index ascending" among ties a
+// warp-local prefix count plus a per-warp base.  One CTA per row; the row stays in L2 between the passes, so
+// HBM sees it once.
+//
+// The histograms avoid a shared-memory atomic per element: those cost about 2 cycles per element and SM whatever
+// the addresses (a first version built on them was ALU-bound, ncu: ALU pipe 72 %, DRAM 5.6 %).  Every LANE of
+// every warp owns private 8-bit counters, lp[warp][bin][lane]: an update is a plain LDS.U8 / IADD / STS.U8 that
+// cannot collide with another lane (one 32-byte row per bin: at most the four lanes of a quad share a bank), and
+// the counters of a warp are folded into 32-bit per-warp totals with DP4A once per 256 elements per lane (an
+// 8-bit counter that wrapped is detected by its owner: after a block the counter of the lane's last element must
+// be non-zero).
+//
+// rq_mine3_kernel (rq_mine3.cuh) is the default selection for rows of 16 384 .. 262 144 values; this kernel
+// finishes the rows it cannot (list mode) and selects rows of any other length.  RQAE_MINE_V2=1, read per call,
+// makes rqae_select_top_middle_bottom_f16 run this kernel for every row, so that the two can be timed and
+// compared in one process; it is the library's only selection switch.
 #pragma once
 #include <cuda_fp16.h>
 
@@ -17,10 +35,6 @@
 
 namespace rq {
 
-constexpr int MN_THREADS = 1024;
-constexpr int MN_WARPS = 32;
-constexpr int MN_BINS = 2048;     // high 11 bits of the descending key
-constexpr int MN_SUB = 32;        // low 5 bits
 constexpr int MN_KMAX = 256;      // largest window
 
 struct MineParams {
@@ -38,251 +52,12 @@ struct MineParams {
   int sample_log2 = 4;    // one 32-byte sector out of 2^sample_log2 is sampled
   int c_top = 24;         // sample count that brackets the top / bottom window
   int c_hi = 0, c_lo = 0; // sample ranks that bracket the middle window
-  unsigned long long* prof = nullptr;   // RQAE_M3_PROF: clocks of steps A / B / C, rows, fallback rows, candidates
 };
 
 // key that sorts ascending when the value sorts descending (+0 just before -0)
 __device__ __forceinline__ uint32_t mn_dkey(uint32_t u) { return (u & 0x8000u) ? u : (~u & 0x7FFFu); }
 __device__ __forceinline__ uint32_t mn_bits(uint32_t d) { return (d & 0x8000u) ? d : (~d & 0x7FFFu); }
 
-struct MineSmem {
-  uint32_t hist1[MN_BINS];                 // counts, then exclusive prefix
-  union {
-    uint32_t hist1b[2][MN_BINS];           // pass 1 only: private copies of the counts (warp % 3 picks hist1 / copy 0 / copy 1)
-    uint32_t hist2[4][MN_WARPS][MN_SUB];   // pass 2
-  };
-  uint32_t scan[MN_WARPS];
-  uint32_t bin[4], rem[4], key[4], less[4];
-  uint32_t base[4][MN_WARPS];
-  uint32_t cnt[3];
-  uint32_t bufk[3][MN_KMAX];
-  uint32_t bufi[3][MN_KMAX];
-};
-
-__global__ void __launch_bounds__(MN_THREADS, 1) rq_mine_kernel(const MineParams p) {
-  __shared__ MineSmem sm;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const long long n = p.n;
-  const int k = p.k, kh = k / 2;
-  const long long seg = ((n + MN_WARPS - 1) / MN_WARPS + 7) / 8 * 8;     // per-warp slice, multiple of 8
-  const long long w_lo = warp * seg, w_hi = (w_lo + seg < n) ? w_lo + seg : n;
-  // descending ranks of the window boundaries: end of top, start / end of middle, start of bottom
-  const long long m0 = n / 2 - kh, m1 = n / 2 + kh;
-  const long long rank[4] = {(long long)k - 1, m0, m1 - 1, n - k};
-
-  for (long long row = blockIdx.x; row < p.rows; row += gridDim.x) {
-    const uint4* src = reinterpret_cast<const uint4*>(p.vals + row * p.row_stride);
-    for (int i = tid; i < 3 * MN_BINS; i += MN_THREADS) sm.hist1[i] = 0;   // hist1 and its two copies are contiguous
-    if (tid < 3) sm.cnt[tid] = 0;
-    __syncthreads();
-
-    // ---- pass 1: histogram of the high 11 key bits ----
-    for (long long i0 = w_lo + lane * 8; i0 < w_hi; i0 += 256) {
-      const uint4 v = __ldg(src + i0 / 8);
-      const uint32_t w4[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-      for (int e = 0; e < 8; e++) {
-        if (i0 + e < w_hi) {
-          const uint32_t d = mn_dkey((w4[e >> 1] >> ((e & 1) * 16)) & 0xFFFFu);
-          atomicAdd(&sm.hist1[(warp % 3) * MN_BINS + (d >> 5)], 1u);
-        }
-      }
-    }
-    __syncthreads();
-    // exclusive prefix over the 2048 bins (2 per thread)
-    {
-      const uint32_t a = sm.hist1[2 * tid] + sm.hist1b[0][2 * tid] + sm.hist1b[1][2 * tid];
-      const uint32_t b = sm.hist1[2 * tid + 1] + sm.hist1b[0][2 * tid + 1] + sm.hist1b[1][2 * tid + 1];
-      uint32_t x = a + b;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
-        if (lane >= o) x += y;
-      }
-      if (lane == 31) sm.scan[warp] = x;
-      __syncthreads();
-      if (warp == 0) {
-        uint32_t t = sm.scan[lane];
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const uint32_t y = __shfl_up_sync(0xffffffffu, t, o);
-          if (lane >= o) t += y;
-        }
-        sm.scan[lane] = t;
-      }
-      __syncthreads();
-      const uint32_t excl = x - (a + b) + (warp > 0 ? sm.scan[warp - 1] : 0u);
-      sm.hist1[2 * tid] = excl;
-      sm.hist1[2 * tid + 1] = excl + a;
-    }
-    __syncthreads();
-    for (int i = tid; i < 4 * MN_WARPS * MN_SUB; i += MN_THREADS) (&sm.hist2[0][0][0])[i] = 0;   // the copies' space is reused
-    if (tid < 4) {   // last bin whose exclusive prefix is <= rank
-      const uint32_t r = (uint32_t)rank[tid];
-      int lo = 0, hi = MN_BINS - 1;
-      while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (sm.hist1[mid] <= r) lo = mid; else hi = mid - 1;
-      }
-      sm.bin[tid] = lo;
-      sm.rem[tid] = r - sm.hist1[lo];
-    }
-    __syncthreads();
-
-    // ---- pass 2: low 5 bits inside the boundary bins, per warp (the per-warp counts give the tie bases) ----
-    {
-      const uint32_t b0 = sm.bin[0], b1 = sm.bin[1], b2 = sm.bin[2], b3 = sm.bin[3];
-      for (long long i0 = w_lo + lane * 8; i0 < w_hi; i0 += 256) {
-        const uint4 v = __ldg(src + i0 / 8);
-        const uint32_t w4[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-        for (int e = 0; e < 8; e++) {
-          if (i0 + e < w_hi) {
-            const uint32_t d = mn_dkey((w4[e >> 1] >> ((e & 1) * 16)) & 0xFFFFu);
-            const uint32_t hb = d >> 5, lb = d & 31u;
-            if (hb == b0) atomicAdd(&sm.hist2[0][warp][lb], 1u);
-            if (hb == b1) atomicAdd(&sm.hist2[1][warp][lb], 1u);
-            if (hb == b2) atomicAdd(&sm.hist2[2][warp][lb], 1u);
-            if (hb == b3) atomicAdd(&sm.hist2[3][warp][lb], 1u);
-          }
-        }
-      }
-    }
-    __syncthreads();
-    if (warp < 4) {   // warp j resolves boundary j: lane = sub-bin
-      const int j = warp;
-      uint32_t c = 0;
-      for (int w = 0; w < MN_WARPS; w++) c += sm.hist2[j][w][lane];
-      uint32_t incl = c;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += y;
-      }
-      const uint32_t rem = sm.rem[j];
-      const bool mine = rem >= incl - c && rem < incl;      // exactly one lane
-      const uint32_t sel = __ballot_sync(0xffffffffu, mine);
-      const int sb = __ffs(sel) - 1;
-      if (mine) {
-        sm.key[j] = (sm.bin[j] << 5) | (uint32_t)lane;
-        sm.less[j] = sm.hist1[sm.bin[j]] + (incl - c);
-      }
-      // tie base of warp `lane`: ties at the boundary key in the warps before it
-      uint32_t t = sm.hist2[j][lane][sb];
-      uint32_t ti = t;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, ti, o);
-        if (lane >= o) ti += y;
-      }
-      sm.base[j][lane] = ti - t;
-    }
-    __syncthreads();
-
-    // ---- pass 3: collect the members of the three windows ----
-    {
-      const uint32_t K0 = sm.key[0], K1 = sm.key[1], K2 = sm.key[2], K3 = sm.key[3];
-      // how many ties at each boundary key fall inside / before the window
-      const uint32_t top_take = (uint32_t)k - sm.less[0];                    // tie ranks < top_take are in top
-      const uint32_t mid_skip = (uint32_t)m0 - sm.less[1];                   // tie ranks >= mid_skip are in middle
-      const uint32_t mid_take = (uint32_t)m1 - sm.less[2];                   // tie ranks < mid_take are in middle
-      const uint32_t bot_skip = (uint32_t)(n - k) - sm.less[3];              // tie ranks >= bot_skip are in bottom
-      uint32_t tc[4] = {sm.base[0][warp], sm.base[1][warp], sm.base[2][warp], sm.base[3][warp]};
-      for (long long i0 = w_lo + lane * 8; i0 - lane * 8 < w_hi; i0 += 256) {   // whole warp iterates together
-        uint32_t d[8];
-        bool live[8];
-        bool cand = false;
-        if (i0 < w_hi) {
-          const uint4 v = __ldg(src + i0 / 8);
-          const uint32_t w4[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-          for (int e = 0; e < 8; e++) {
-            live[e] = i0 + e < w_hi;
-            d[e] = mn_dkey((w4[e >> 1] >> ((e & 1) * 16)) & 0xFFFFu);
-            // inside or on the edge of a window (an element equal to a boundary key always is)
-            cand |= live[e] && (d[e] <= K0 || d[e] >= K3 || (d[e] >= K1 && d[e] <= K2));
-          }
-        } else {
-#pragma unroll
-          for (int e = 0; e < 8; e++) { live[e] = false; d[e] = 0; }
-        }
-        if (!__any_sync(0xffffffffu, cand)) continue;
-        uint32_t neq[4] = {0, 0, 0, 0};
-#pragma unroll
-        for (int e = 0; e < 8; e++) {
-          if (live[e]) { neq[0] += d[e] == K0; neq[1] += d[e] == K1; neq[2] += d[e] == K2; neq[3] += d[e] == K3; }
-        }
-        // tie ranks: exclusive prefix over the lanes of the per-lane tie counts, per boundary key
-        uint32_t ex[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-          uint32_t x = neq[j];
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= o) x += y;
-          }
-          ex[j] = tc[j] + x - neq[j];
-          tc[j] += __shfl_sync(0xffffffffu, x, 31);
-        }
-        if (cand) {
-#pragma unroll
-          for (int e = 0; e < 8; e++) {
-            if (!live[e]) continue;
-            const uint32_t dd = d[e];
-            const uint32_t t0 = ex[0], t1 = ex[1], t2 = ex[2], t3 = ex[3];
-            ex[0] += dd == K0; ex[1] += dd == K1; ex[2] += dd == K2; ex[3] += dd == K3;
-            const bool in_top = dd < K0 || (dd == K0 && t0 < top_take);
-            const bool in_mid = kh > 0 && (dd > K1 || (dd == K1 && t1 >= mid_skip)) && (dd < K2 || (dd == K2 && t2 < mid_take));
-            const bool in_bot = dd > K3 || (dd == K3 && t3 >= bot_skip);
-            const uint32_t index = (uint32_t)(i0 + e);
-            if (in_top) { const uint32_t s = atomicAdd(&sm.cnt[0], 1u); if (s < MN_KMAX) { sm.bufk[0][s] = dd; sm.bufi[0][s] = index; } }
-            if (in_mid) { const uint32_t s = atomicAdd(&sm.cnt[1], 1u); if (s < MN_KMAX) { sm.bufk[1][s] = dd; sm.bufi[1][s] = index; } }
-            if (in_bot) { const uint32_t s = atomicAdd(&sm.cnt[2], 1u); if (s < MN_KMAX) { sm.bufk[2][s] = dd; sm.bufi[2][s] = index; } }
-          }
-        }
-      }
-    }
-    __syncthreads();
-
-    // ---- order each window by (key, index) and write it out ----
-    for (int w = 0; w < 3; w++) {
-      const int cnt = min((int)sm.cnt[w], MN_KMAX);
-      int* io = p.idx_out + (row * 3 + w) * (long long)k;
-      __half* vo = p.val_out ? p.val_out + (row * 3 + w) * (long long)k : nullptr;
-      if (tid < cnt) {
-        const uint32_t dk = sm.bufk[w][tid], di = sm.bufi[w][tid];
-        int r = 0;
-        for (int o = 0; o < cnt; o++) {
-          const uint32_t ok = sm.bufk[w][o], oi = sm.bufi[w][o];
-          r += (ok < dk) || (ok == dk && oi < di);
-        }
-        if (r < k) {
-          io[r] = (int)di;
-          if (vo) vo[r] = __ushort_as_half((unsigned short)mn_bits(dk));
-        }
-      } else if (tid < k) {
-        // slots beyond the window's size (odd k: the middle window holds k - 1 values)
-        if (tid >= cnt) { io[tid] = -1; if (vo) vo[tid] = __ushort_as_half((unsigned short)0); }
-      }
-    }
-    __syncthreads();
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// rq_mine2_kernel: the same selection, the same total order and the same three passes, without a shared-memory
-// atomic per element.  The first version spent its time in ATOMS (ncu: ALU pipe 72 %, DRAM 5.6 %: 2 cycles per
-// element and SM whatever the addresses).  Here a histogram digit is 8 bits and every LANE of every warp owns
-// private 8-bit counters, lp[warp][bin][lane]: an update is a plain LDS.U8 / IADD / STS.U8 that cannot collide
-// with another lane (one 32-byte row per bin: at most the four lanes of a quad share a bank), and the counters of
-// a warp are folded into 32-bit per-warp totals with DP4A once per 256 elements per lane (an 8-bit counter that
-// wrapped is detected by its owner: after a block the counter of the lane's last element must be non-zero).
-//   pass 1  histogram of the high key byte (raw bit pattern; bins are visited in descending-value order later)
-//   pass 2  histogram of the low byte inside the bin that holds the median window (lane-private again); the bins
-//           that hold the top / bottom boundaries are tails with few members and use per-warp atomics
-//   pass 3  collects the members of the three windows (identical to the first version)
-// One CTA of 512 threads per row, 200 KB of shared memory, one CTA per SM.
 #ifndef RQ_M2_WARPS
 #define RQ_M2_WARPS 8   /* 8: two CTAs per SM (one row's serial steps run under the other's streaming); 16: one CTA per SM */
 #endif

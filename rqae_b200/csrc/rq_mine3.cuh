@@ -101,7 +101,6 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
   for (long long row = blockIdx.x; row < p.rows; row += gridDim.x) {
     const uint4* src = reinterpret_cast<const uint4*>(p.vals + row * p.row_stride);
     const unsigned short* src16 = reinterpret_cast<const unsigned short*>(p.vals + row * p.row_stride);
-    const long long t0 = clock64();
     for (int i = tid; i < M3_BINS; i += M3_THREADS) sm.hist[0][i] = 0;
     if (tid < 128) (&sm.h2[0][0][0])[tid] = 0;
     if (tid == 0) {
@@ -204,7 +203,6 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
     // ---- B: one pass over the row ----
     // A NaN compares "greater or unordered" to T_top, so it becomes a candidate; step C sees its bit pattern and sends
     // the row to the fallback (no separate NaN test per value).
-    const long long t1 = clock64();
     {
       uint32_t gcount = 0;
       uint32_t gacc = 0;                                              // 510 x (values above the bracket)
@@ -330,7 +328,6 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
     // m1 - 1 - G;  class 2: values <= T_bot, window = its last k.  Per class a two-level radix select over the key
     // range [kbase, kend] (+0 / -0 compare equal: a range that ends at one of them is widened over both), then a rank
     // sort of the keys that remain.
-    const long long t2 = clock64();
     if (row + gridDim.x < p.rows) {   // the next row of this CTA: sample sectors and the first chunks on their way to L2
       const long long nrow = row + gridDim.x;
       const uint4* nsrc = reinterpret_cast<const uint4*>(p.vals + nrow * p.row_stride);
@@ -344,15 +341,9 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
       }
     }
     const uint32_t G = sm.G;
-    uint32_t ncand = 0;
     bool ok = true;
 #pragma unroll
-    for (int w = 0; w < M3_WARPS; w++) {
-      const uint32_t cw = sm.wcount[w];
-      ncand += cw;
-      ok = ok && cw <= (uint32_t)M3_WCAP;
-    }
-    uint32_t why = ok ? 0u : 1u;   // RQAE_M3_PROF: 1 region overflow, 2 NaN, 4 bracket missed, 8 tail class short, 16 a warp's short list of window-range keys overflowed
+    for (int w = 0; w < M3_WARPS; w++) ok = ok && sm.wcount[w] <= (uint32_t)M3_WCAP;
     // this warp's candidates: slots wb .. wb + wn
     const uint32_t wb = (uint32_t)warp * M3_WCAP, wn = ok ? sm.wcount[warp] : 0u;
     // C1: level-1 histograms of the two tail classes (the buffer holds keys; NaN keys lie beyond the two infinities)
@@ -371,9 +362,7 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
       }
     }
     __syncthreads();
-    if (sm.nan != 0) why |= 2u;
     ok = ok && sm.nan == 0;
-    const long long tc1 = clock64();
     // C2: prefix sums, the bins of each window's first and last rank
     uint32_t rl0 = 0, rl1 = 0, rl2 = 0, rh0 = 0, rh1 = 0, rh2 = 0;
     {
@@ -399,11 +388,11 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
         uint32_t rl, rh;
         if (c == 1) {
           if (kh == 0) continue;
-          if ((long long)G > m0 || (long long)G + (long long)total < m1) { ok = false; why |= 4u; continue; }
+          if ((long long)G > m0 || (long long)G + (long long)total < m1) { ok = false; continue; }
           rl = (uint32_t)(m0 - (long long)G); rh = (uint32_t)(m1 - 1 - (long long)G);
           rl1 = rl; rh1 = rh;
         } else {
-          if (total < (uint32_t)k) { ok = false; why |= 8u; continue; }
+          if (total < (uint32_t)k) { ok = false; continue; }
           rl = c == 0 ? 0u : total - (uint32_t)k; rh = rl + (uint32_t)k - 1u;
           if (c == 0) { rl0 = rl; rh0 = rh; } else { rl2 = rl; rh2 = rh; }
         }
@@ -417,8 +406,6 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
       }
     }
     __syncthreads();
-    const long long tc2 = clock64();
-    long long tc3 = tc2, tc4 = tc2, tc5 = tc2;
     if (ok) {   // block-uniform
       // C3: the low key bits inside the boundary bins (first key of bin A / B of each class)
       const uint32_t fa0 = kb0 + (sm.binA[0] << sh0), fb0 = kb0 + (sm.binB[0] << sh0);
@@ -450,7 +437,6 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
         }
         __syncthreads();
       }
-      tc3 = clock64();
       // C4: warp 2 c + b resolves boundary b of class c
       if (warp < 6) {
         const int c = warp >> 1, b = warp & 1;
@@ -472,7 +458,6 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
         }
       }
       __syncthreads();
-      tc4 = clock64();
       // C5: the members of the three windows.  A key strictly between the boundary keys is in; a key EQUAL to a boundary
       // key is in according to its rank among the equal values in index order: regions are in index order (step B), so
       // that rank is (equal values in earlier warps' regions) + (equal values earlier in this region).
@@ -520,7 +505,7 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
         if (lane == 0 && nsl > SL) sm.nan = 2u;   // the short list overflowed (a tie group of thousands): the row falls back
       }
       __syncthreads();
-      if (sm.nan != 0) { ok = false; why |= 16u; }
+      if (sm.nan != 0) ok = false;
       uint32_t run[6];                                  // equal values before the current position (warp-uniform)
       {   // lane w holds the counts of warp w, two keys per word; the warps before this one are summed
         uint32_t pk[3];
@@ -573,9 +558,8 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
       }
       __syncthreads();
       if (sm.lcount[0] > (uint32_t)M3_LIST || sm.lcount[2] > (uint32_t)M3_LIST || (kh > 0 && sm.lcount[1] > (uint32_t)M3_LIST)) {
-        ok = false; why |= 16u;   // cannot happen: a list holds exactly its window
+        ok = false;   // cannot happen: a list holds exactly its window
       }
-      tc5 = clock64();
       if (ok) {
         // C6: rank sorts, five warps per class: packed (key, index) ascending = value descending, index ascending
         const int c = tid / M3_SORT_THREADS;
@@ -617,23 +601,6 @@ __global__ void __launch_bounds__(M3_THREADS, 2) rq_mine3_kernel(const MineParam
       p.fb_list[slot] = (int)row;
     }
     __syncthreads();
-    if (p.prof && tid == 0) {
-      const long long t3 = clock64();
-      atomicAdd(p.prof + 0, (unsigned long long)(t1 - t0));
-      atomicAdd(p.prof + 1, (unsigned long long)(t2 - t1));
-      atomicAdd(p.prof + 2, (unsigned long long)(t3 - t2));
-      atomicAdd(p.prof + 3, 1ull);
-      atomicAdd(p.prof + 4, ok ? 0ull : 1ull);
-      atomicAdd(p.prof + 5, (unsigned long long)ncand);
-      atomicAdd(p.prof + 6, (unsigned long long)(tc1 - t2));
-      atomicAdd(p.prof + 7, (unsigned long long)(tc2 - tc1));
-      atomicAdd(p.prof + 8, (unsigned long long)(tc3 - tc2));
-      atomicAdd(p.prof + 9, (unsigned long long)(tc4 - tc3));
-      atomicAdd(p.prof + 10, (unsigned long long)(tc5 - tc4));
-      atomicAdd(p.prof + 11, (unsigned long long)(t3 - tc5));
-      for (int bit = 0; bit < 5; bit++)
-        if (why & (1u << bit)) atomicAdd(p.prof + 12 + bit, 1ull);
-    }
   }
 }
 

@@ -19,7 +19,7 @@
 //                             <= 64 layers (ascending layer order), one rounding to fp16 per chunk, chunks
 //                             of a range added in fp16 (server.py:216-234), ranges added in fp16 (:256-259)
 //   search_posmax_kernel      max over the S positions of every dataset sequence (server.py:265-267),
-//                             written query-position-major so that rq_mine_kernel (rq_mine.cuh) can rank the
+//                             written query-position-major so that the selection (rq_mine.cuh) can rank the
 //                             sequences of every query position without the reference's full argsort
 //
 // Bound: the table rows.  A token-layer reads 256 B of table against 2-4 B of code store, and a layer's slab
@@ -91,12 +91,13 @@ __device__ __forceinline__ uint32_t sr_pack(float a, float b) {
 }
 __device__ __forceinline__ float2 sr_unpack(uint32_t w) { return __half22float2(*reinterpret_cast<const __half2*>(&w)); }
 
-// DEPTH = layers of row loads kept in flight per token: the loads of layer i + DEPTH are issued as soon as layer i has
-// been consumed (DEPTH x 8 independent 256-byte rows outstanding per warp).  Measured on the whole store, DEPTH 1 / 2 / 3
-// = 197 / 196 / 275 ms: the kernel is bound by what L2 delivers, not by the latency a warp sees, so 2 is the default
-// (it rides out the DRAM misses of the longest range) and 3 only adds queueing.
-template <typename CodeT, int DEPTH>
+template <typename CodeT>
 __global__ void __launch_bounds__(SR_THREADS, 2) search_accumulate_kernel(const SearchAccParams p) {
+  // DEPTH = layers of row loads kept in flight per token: the loads of layer i + DEPTH are issued as soon as layer i
+  // has been consumed (DEPTH x 8 independent 256-byte rows outstanding per warp).  Measured on the whole store,
+  // DEPTH 1 / 2 / 3 = 197 / 196 / 275 ms (profiles/r1s_search_ab.jsonl): the kernel is bound by what L2 delivers, not
+  // by the latency a warp sees, so 2 rides out the DRAM misses of the longest range and 3 only adds queueing.
+  constexpr int DEPTH = 2;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const CodeT* __restrict__ codes = (const CodeT*)p.codes;
   const long long n_tiles = (p.n_tokens + SR_TILE - 1) / SR_TILE;

@@ -2,7 +2,6 @@
 // launch.  Host logic only; the kernels live in rq_forward.cuh / rq_decode.cuh.
 #include <cuda.h>
 #include <cuda_runtime.h>
-#include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -382,8 +381,7 @@ int launch_forward_t(const rq::FwdParams& prm, int sms, cudaStream_t st) {
   const int grid = (int)(n_units < sms ? n_units : sms);
   rq::FwdParams p2 = prm;
   p2.sync_ctr = nullptr;
-  static const bool lockstep = [] { const char* e = getenv("RQAE_LOCKSTEP"); return e ? atoi(e) != 0 : true; }();
-  if (lockstep && n_units > grid) {
+  if (n_units > grid) {
     // more than one unit per CTA: keep the CTAs' weight streams in step (one counter per launch in flight).
     // The kernel spins on the counter, so all CTAs must be co-resident: cooperative launch guarantees it.
     unsigned int* base = nullptr;
@@ -440,8 +438,7 @@ int launch_forward_cluster_t(const rq::FwdParams& prm, int sms, cudaStream_t st)
   const int clusters = (int)(n_units < ncl ? n_units : ncl);
   rq::FwdParams p2 = prm;
   p2.sync_ctr = nullptr;
-  static const bool lockstep = [] { const char* e = getenv("RQAE_LOCKSTEP"); return e ? atoi(e) != 0 : true; }();
-  const bool coop = lockstep && n_units > clusters;
+  const bool coop = n_units > clusters;
   if (coop) {
     unsigned int* base = nullptr;
     RQ_CUDA(cudaGetSymbolAddress((void**)&base, g_sync_ctr));
@@ -571,21 +568,13 @@ static int forward_common(const void* packed, const float* codebook, int codeboo
   prm.off_tp = L.off_tp; prm.off_map3 = L.off_map3;
   prm.codebook = codebook; prm.cb_shared = codebook_shared ? 1 : 0; prm.K = K; prm.nq_run = nq_run; prm.D = dim;
   prm.n_tokens = n_tokens; prm.codes = codes; prm.code_dtype = code_dtype; prm.code_stride = code_stride;
-  {
-    static const float l2_hot = [] {   // tuning knob (DESIGN.md, "L2 residency of the weight stream")
-      const char* e = getenv("RQAE_L2_HOT");
-      const float v = e ? (float)atof(e) : RQ_L2_HOT_DEFAULT;
-      return v < 0.0f ? 0.0f : (v > 1.0f ? 1.0f : v);
-    }();
-    prm.l2_hot = l2_hot;
-  }
+  prm.l2_hot = RQ_L2_HOT_DEFAULT;   // DESIGN.md, "L2 residency of the weight stream"
   cudaStream_t st = (cudaStream_t)stream;
   // Few tokens (the hook's operating point is 4 x 128, scripts/1_create_activations.py:152): units of 2 x 4 tokens
   // instead of 2 x 8 put twice as many SMs to work and halve the time of a pass; a token's arithmetic does not
   // depend on the unit size, so the codes are the same bit for bit.  (Units of 2 x 2 would ask the L2 for more
-  // weight bytes per layer than it delivers.)  RQAE_SMALL_UNITS=0 switches it off (A/B timing).
-  static const bool small_units = [] { const char* e = getenv("RQAE_SMALL_UNITS"); return e ? atoi(e) != 0 : true; }();
-  const bool few = small_units && n_tokens <= (int64_t)sms * 8;
+  // weight bytes per layer than it delivers.)
+  const bool few = n_tokens <= (int64_t)sms * 8;
   switch (s.E) {
     case 1: return launch_forward<1, 1, 1, 4, 8>(prm, sms, st);
     case 3: return launch_forward<3, 3, 1, 4, 8>(prm, sms, st);
@@ -1074,12 +1063,6 @@ static int int_layout(const int32_t* cuts, int n_cuts, int F, int64_t n_tokens, 
   return RQAE_OK;
 }
 
-int rqae_intensity_profile(uint64_t* out_host, int n_ctas) {
-  if (!out_host || n_ctas <= 0 || n_ctas > 256) return RQAE_EINVAL;
-  RQ_CUDA(cudaMemcpyFromSymbol(out_host, rq::g_int_prof, (size_t)n_ctas * rq::IT_PROF_SLOTS * sizeof(unsigned long long)));
-  return RQAE_OK;
-}
-
 static long long ip_units(const IntLayout& L) { return (L.T_pad / rq::IT_TOK) * (long long)((L.F_tiles + 1) / 2); }
 
 size_t rqae_intensity_workspace_bytes(const int32_t* cuts_host, int n_cuts, int n_features, int64_t n_tokens) {
@@ -1159,11 +1142,9 @@ static int intensity_impl(const float* cb_norm, int K, const void* codes, int co
   ip.codes_p = (const uint32_t*)(ws + L.off_codes); ip.L = L.L; ip.T_pad = L.T_pad; ip.u_tiles = ws + L.off_u;
   ip.sched = (const rq::IntKBlock*)(ws + L.off_sched); ip.wcum = (const float*)(ws + L.off_wcum);
   ip.lut = (const uint2*)(ws + L.off_lut); ip.K = K; ip.NKB = L.NKB; ip.n_cuts = n_cuts; ip.F = n_features;
-  { const char* e = getenv("RQAE_INT_DBG"); ip.dbg = e ? atoi(e) : 0; }
   const long long units = ip_units(L);
-  // start groups 20 k clocks apart when every CTA has several units to run (RQAE_INT_STAGGER overrides, for experiments)
-  { const char* e = getenv("RQAE_INT_STAGGER"); ip.stagger = e ? atoi(e) : (units >= 4LL * sms && n_cuts >= 4 ? 20000 : 0); }
-  { const char* e = getenv("RQAE_INT_GROUPS"); ip.stagger_groups = e && atoi(e) > 0 ? atoi(e) : 4; }
+  // start groups 20 k clocks apart when every CTA has several units to run
+  ip.stagger = units >= 4LL * sms && n_cuts >= 4 ? 20000 : 0;
   ip.q_out = nullptr; ip.bias = nullptr; ip.T = n_tokens; ip.D = 0;
   ip.F_tiles = L.F_tiles; ip.out = (__half*)out; ip.out_stride = out_stride; ip.n_tok_tiles = L.T_pad / rq::IT_TOK;
   const int grid = (int)(units < sms ? units : sms);
@@ -1189,19 +1170,19 @@ int rqae_select_top_middle_bottom_f16(const void* vals, int64_t rows, int64_t ro
   rq::MineParams mp;
   mp.vals = (const __half*)vals; mp.rows = rows; mp.row_stride = row_stride; mp.n = n; mp.k = top_k;
   mp.idx_out = idx_out; mp.val_out = (__half*)val_out;
-  // RQAE_MINE_V1=1 selects the first version of the kernel (shared-memory atomics per element; A/B timing)
-  static const bool v1 = [] { const char* e = getenv("RQAE_MINE_V1"); return e && atoi(e) != 0; }();
   // RQAE_MINE_V2=1 keeps the three-pass kernel for every row (A/B timing against the sample-bracketed one)
   const bool v2 = [] { const char* e = getenv("RQAE_MINE_V2"); return e && atoi(e) != 0; }();   // read per call: A/B in one process
   constexpr int smem2 = rq::M2_SMEM_BYTES_PAD + rq::M2_LP_BYTES + (int)sizeof(rq::Mine2Smem);
   constexpr int per_sm2 = 16 / rq::M2_WARPS;
-  if (!v1 && !v2 && n >= 16384 && n <= 262144 && rows < ((int64_t)1 << 31)) {
+  static_assert(smem2 <= (228 * 1024 - per_sm2 * 1024) / per_sm2, "shared memory budget");
+  if (!v2 && n >= 16384 && n <= 262144 && rows < ((int64_t)1 << 31)) {
     // rq_mine3_kernel: brackets from a sample, one streaming pass, exact selection among the candidates; rows whose
     // brackets miss are finished by rq_mine2_kernel in list mode
     const int slog = n <= 131072 ? 4 : 3;
     const double ms = (double)(((n / 16) >> slog) * 16), s = (double)n / ms, sig = 0.5 * sqrt(ms);
-    // half-width of the median bracket in sigmas of the sample's rank error (RQAE_M3_Z overrides, for experiments)
-    const double z = [] { const char* e = getenv("RQAE_M3_Z"); const double v = e ? atof(e) : 0.0; return v >= 1.0 && v <= 8.0 ? v : 4.0; }();
+    // half-width of the median bracket in sigmas of the sample's rank error (sweep of 4.5 / 4 / 3.5 / 3:
+    // profiles/r5z_select_z_sweep.txt)
+    constexpr double z = 4.0;
     const long long kh = top_k / 2, m0 = n / 2 - kh, m1 = n / 2 + kh;
     mp.sample_log2 = slog;
     mp.c_top = (int)ceil(top_k / s + 6.0 * sqrt(top_k / s) + 3.0);
@@ -1214,9 +1195,6 @@ int rqae_select_top_middle_bottom_f16(const void* vals, int64_t rows, int64_t ro
     cudaError_t e = cudaMemsetAsync(fb, 0, sizeof(int), st);
     if (e == cudaSuccess) {
       mp.fb_count = fb; mp.fb_list = fb + 1;
-      static const bool prof = [] { const char* pe = getenv("RQAE_M3_PROF"); return pe && atoi(pe) != 0; }();
-      unsigned long long* dprof = nullptr;
-      if (prof && cudaMalloc((void**)&dprof, 256) == cudaSuccess) { cudaMemset(dprof, 0, 256); mp.prof = dprof; }
       constexpr int smem3 = (int)sizeof(rq::Mine3Smem);
       static_assert(2 * (smem3 + 1024) <= 227 * 1024, "two CTAs per SM");
       e = ensure_dynamic_smem((const void*)rq::rq_mine3_kernel, smem3);
@@ -1224,20 +1202,6 @@ int rqae_select_top_middle_bottom_f16(const void* vals, int64_t rows, int64_t ro
         const int grid = (int)(rows < 2LL * sms ? rows : 2LL * sms);
         rq::rq_mine3_kernel<<<grid, rq::M3_THREADS, smem3, st>>>(mp);
         e = cudaGetLastError();
-        if (dprof) {   // timing experiment only: synchronises
-          unsigned long long h[32] = {0};
-          cudaStreamSynchronize(st);
-          cudaMemcpy(h, dprof, 256, cudaMemcpyDeviceToHost);
-          cudaFree(dprof);
-          mp.prof = nullptr;
-          const double r = h[3] ? (double)h[3] : 1.0;
-          fprintf(stderr, "rq_mine3 clocks per row: sample %.0f, stream %.0f, select %.0f; rows %llu, fallback %llu, candidates per row %.0f\n",
-                  h[0] / r, h[1] / r, h[2] / r, h[3], h[4], h[5] / r);
-          fprintf(stderr, "  select steps: histogram %.0f, prefix %.0f, low bits %.0f, resolve %.0f, collect %.0f, rank sort %.0f\n",
-                  h[6] / r, h[7] / r, h[8] / r, h[9] / r, h[10] / r, h[11] / r);
-          if (h[4]) fprintf(stderr, "  fallback reasons: region overflow %llu, NaN %llu, bracket missed %llu, tail class short %llu, short list overflow %llu\n",
-                            h[12], h[13], h[14], h[15], h[16]);
-        }
       }
       if (e == cudaSuccess) e = ensure_dynamic_smem((const void*)rq::rq_mine2_kernel, smem2);
       if (e == cudaSuccess) {
@@ -1253,17 +1217,9 @@ int rqae_select_top_middle_bottom_f16(const void* vals, int64_t rows, int64_t ro
     g_launches += 2;
     return RQAE_OK;
   }
-  if (v1) {
-    const int grid = (int)(rows < 2LL * sms ? rows : 2LL * sms);
-    rq::rq_mine_kernel<<<grid, rq::MN_THREADS, 0, (cudaStream_t)stream>>>(mp);
-  } else {
-    constexpr int smem = smem2;
-    constexpr int per_sm = per_sm2;
-    static_assert(smem <= (228 * 1024 - per_sm * 1024) / per_sm, "shared memory budget");
-    RQ_CUDA(ensure_dynamic_smem((const void*)rq::rq_mine2_kernel, smem));
-    const int grid = (int)(rows < (long long)sms * per_sm ? rows : (long long)sms * per_sm);
-    rq::rq_mine2_kernel<<<grid, rq::M2_THREADS, smem, (cudaStream_t)stream>>>(mp);
-  }
+  RQ_CUDA(ensure_dynamic_smem((const void*)rq::rq_mine2_kernel, smem2));
+  const int grid = (int)(rows < (long long)sms * per_sm2 ? rows : (long long)sms * per_sm2);
+  rq::rq_mine2_kernel<<<grid, rq::M2_THREADS, smem2, st>>>(mp);
   RQ_CUDA(cudaGetLastError());
   g_launches++;
   return RQAE_OK;
@@ -1312,19 +1268,9 @@ int rqae_search_accumulate_f16(const void* table, int K, const void* codes, int 
   const long long tiles = (n_tokens + rq::SR_TILE - 1) / rq::SR_TILE;
   const int grid = (int)(tiles < 4LL * sms ? tiles : 4LL * sms);
   cudaStream_t st = (cudaStream_t)stream;
-  // RQAE_SEARCH_DEPTH = 1 / 2 / 3 selects how many layers of row loads a warp keeps in flight (A/B timing knob;
-  // measured on the full store: 197 / 196 / 275 ms, profiles/r1s_search_ab.jsonl)
-  static const int depth = [] { const char* e = getenv("RQAE_SEARCH_DEPTH"); const int d = e ? atoi(e) : 2; return d < 1 ? 1 : (d > 3 ? 3 : d); }();
-#define RQ_SR_LAUNCH(T)                                                                                   \
-  do {                                                                                                    \
-    if (depth == 1) rq::search_accumulate_kernel<T, 1><<<grid, rq::SR_THREADS, 0, st>>>(ap);              \
-    else if (depth == 2) rq::search_accumulate_kernel<T, 2><<<grid, rq::SR_THREADS, 0, st>>>(ap);         \
-    else rq::search_accumulate_kernel<T, 3><<<grid, rq::SR_THREADS, 0, st>>>(ap);                         \
-  } while (0)
-  if (code_dtype == RQAE_CODE_I64) RQ_SR_LAUNCH(long long);
-  else if (code_dtype == RQAE_CODE_I32) RQ_SR_LAUNCH(int);
-  else RQ_SR_LAUNCH(short);
-#undef RQ_SR_LAUNCH
+  if (code_dtype == RQAE_CODE_I64) rq::search_accumulate_kernel<long long><<<grid, rq::SR_THREADS, 0, st>>>(ap);
+  else if (code_dtype == RQAE_CODE_I32) rq::search_accumulate_kernel<int><<<grid, rq::SR_THREADS, 0, st>>>(ap);
+  else rq::search_accumulate_kernel<short><<<grid, rq::SR_THREADS, 0, st>>>(ap);
   RQ_CUDA(cudaGetLastError());
   g_launches++;
   return RQAE_OK;
@@ -1334,7 +1280,7 @@ int rqae_search_position_max_f16(const void* acc, int64_t n_seq, int seq_len, in
                                  int64_t out_stride, void* stream) {
   if (!acc || !out || n_seq < 0 || seq_len <= 0 || n_query <= 0) return RQAE_EINVAL;
   if (n_query > rq::SR_Q) return RQAE_EUNSUPPORTED;
-  if (out_stride < n_seq || (out_stride & 7) || ((uintptr_t)out & 15)) return RQAE_EINVAL;   // the layout rq_mine_kernel reads
+  if (out_stride < n_seq || (out_stride & 7) || ((uintptr_t)out & 15)) return RQAE_EINVAL;   // the layout rqae_select_top_middle_bottom_f16 reads
   if ((uintptr_t)acc & 7) return RQAE_EINVAL;                                                // 8-byte lane loads
   if (out_stride == 0) return RQAE_OK;
   int sms = 0;
@@ -1448,8 +1394,7 @@ int rqae_search_tc_maxima_f16(const void* store_tc, int64_t n_seq, int seq_len, 
   ip.u_tiles = ws + 4096; ip.sched = (const rq::IntKBlock*)ws; ip.K = K; ip.NKB = nkb; ip.n_cuts = n_layers_list;
   ip.F = n_query; ip.F_tiles = 1; ip.n_tok_tiles = units; ip.L = last; ip.T_pad = units * rq::IT_TOK;
   ip.s_codes = (const uint4*)store_tc; ip.s_vtab = (const uint4*)vtab_f16; ip.s_max = (__half*)max_out;
-  ip.s_stride = max_stride; ip.s_len = seq_len; ip.L8 = L8; ip.stagger = 0; ip.stagger_groups = 1;
-  { const char* e = getenv("RQAE_INT_DBG"); ip.dbg = e ? atoi(e) : 0; }
+  ip.s_stride = max_stride; ip.s_len = seq_len; ip.L8 = L8; ip.stagger = 0;
   const int grid = (int)(units < sms ? units : sms);
   CUtensorMap no_map;
   memset(&no_map, 0, sizeof(no_map));
@@ -1586,8 +1531,7 @@ int rqae_decode_tc_f32(const float* w_out, const float* b_out, const float* code
   ip.sched = (const rq::IntKBlock*)(ws + L.off_sched); ip.wcum = (const float*)(ws + L.off_wcum);
   ip.lut = (const uint2*)(ws + L.off_lut); ip.K = K; ip.NKB = L.NKB; ip.n_cuts = 1; ip.F = dim; ip.F_tiles = L.F_tiles;
   ip.n_tok_tiles = L.T_pad / rq::IT_TOK; ip.q_out = q_out; ip.bias = (const float*)(ws + L.off_bias); ip.T = n_tokens; ip.D = dim;
-  { const char* e = getenv("RQAE_INT_DBG"); ip.dbg = e ? atoi(e) : 0; }
-  ip.stagger = 0; ip.stagger_groups = 1;
+  ip.stagger = 0;
   const long long units = ip.n_tok_tiles * ((L.F_tiles + 1) / 2);
   const int grid = (int)(units < sms ? units : sms);
   CUtensorMap no_map;

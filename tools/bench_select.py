@@ -24,5 +24,5 @@ for _ in range(a.reps):
     idx, val = select_top_middle_bottom(v, 100)
 e1.record(); torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / a.reps
-print(f"select {'v1' if os.environ.get('RQAE_MINE_V1') == '1' else 'v2' if os.environ.get('RQAE_MINE_V2') == '1' else 'v3'}: rows {a.rows} n {a.n}: {ms:.3f} ms, "
+print(f"select {'v2' if os.environ.get('RQAE_MINE_V2') == '1' else 'v3'}: rows {a.rows} n {a.n}: {ms:.3f} ms, "
       f"{a.rows * a.n * 2 / ms / 1e6:.1f} GB/s of row bytes, checksum {int(idx.long().sum().item())}")

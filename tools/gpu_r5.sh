@@ -11,8 +11,7 @@ timeout 1200 python -m pytest tests -m gpu -x -q 2>&1 | tail -4 | tee $OUT/pytes
 echo "=== smoke ==="
 timeout 300 python -c "import __graft_entry__ as g; g.smoke()" 2>&1 | tail -2 | tee $OUT/smoke_$TAG.log
 echo "=== selection A/B (normal rows) ==="
-{ RQAE_M3_PROF=1 timeout 120 python tools/bench_select.py --reps 1 2>&1 | tail -3
-  for v in 0 1; do RQAE_MINE_V2=$v timeout 120 python tools/bench_select.py 2>&1 | tail -1; done; } | tee $OUT/select_ab_$TAG.log
+for v in 0 1; do RQAE_MINE_V2=$v timeout 120 python tools/bench_select.py 2>&1 | tail -1; done | tee $OUT/select_ab_$TAG.log
 echo "=== bench ==="
 timeout 900 python bench.py --steps 5 --warmup 3 > $OUT/bench_$TAG.json 2> $OUT/bench_$TAG.err; echo "bench exit=$?"
 tail -3 $OUT/bench_$TAG.err

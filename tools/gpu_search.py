@@ -78,7 +78,7 @@ def bench(N, S=127, nq=1024, K=625, Sq=127, reps=2):
     # property at full size: the query sequence is the top example of each of its own positions at the last layer
     self_top = bool((sel[:, 0, 0] == idx).all().item())
     rows = N * S * max(layers)
-    emit(what="search_bench", depth=os.environ.get("RQAE_SEARCH_DEPTH", "default"), sequences=N, positions=S, layers=max(layers), query_positions=Sq, K=K,
+    emit(what="search_bench", sequences=N, positions=S, layers=max(layers), query_positions=Sq, K=K,
          total_ms=round(best["total_ms"], 3), wall_ms=round(best["wall_ms"], 3), launches=best["launches"],
          sequences_per_s=round(N / (best["total_ms"] * 1e-3), 1),
          table_row_TBps=round(rows * 256 / (best["total_ms"] * 1e-3) / 1e12, 3),
@@ -93,8 +93,7 @@ def main():
     if "--no-tests" not in sys.argv:
         import pytest
         rc = pytest.main(["-x", "-q", "-m", "gpu", os.path.join(ROOT, "tests", "test_search_gpu.py"), "-p", "no:cacheprovider"])
-        emit(what="pytest tests/test_search_gpu.py", exit_code=int(rc), seconds=round(time.time() - t0, 1),
-             depth=os.environ.get("RQAE_SEARCH_DEPTH", "default"))
+        emit(what="pytest tests/test_search_gpu.py", exit_code=int(rc), seconds=round(time.time() - t0, 1))
         if int(rc) != 0:
             return int(rc)
     if "--bench-extra" in sys.argv:        # the exact function bench.py runs as extra["example_search"], on the 2B model

@@ -1,5 +1,5 @@
 """Selection on the intensity GEMM's own rows, cut by cut: time of the sample-bracketed kernel and of the three-pass
-kernel, and (RQAE_M3_PROF=1) how many rows fell back.  usage: RQAE_M3_PROF=1 python tools/select_gemm_rows.py"""
+kernel.  usage: python tools/select_gemm_rows.py"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
