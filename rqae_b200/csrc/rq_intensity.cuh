@@ -703,10 +703,11 @@ __global__ void int_prep_kernel(const IntPrepParams p) {
 // codes [T][stride] (int16 / int32 / int64) -> tile-major int16 pairs [T_pad/256][L][128][2]: within a tile of 256
 // tokens the codes of token b and token b+128 at one layer share a 32-bit word (the two rows one builder thread
 // writes), and a tile's layers are contiguous (one bulk L2 prefetch per K-block).  Out-of-range codes and the
-// padding tokens map to K (the zero row of the lookup table).
+// padding tokens map to K (the zero row of the lookup table).  wrap_negative (decode): a code in [-K, 0) first takes the
+// python-style index c + K, as codebook[0][codes] and the bit-exact decode do.
 template <typename CT>
 __global__ void __launch_bounds__(256) int_transpose_kernel(const CT* __restrict__ codes, long long stride, long long T, int L,
-                                                            int K, uint32_t* __restrict__ out) {
+                                                            int K, bool wrap_negative, uint32_t* __restrict__ out) {
   // block = one token tile (256 tokens) x 32 layers, staged in shared memory as [token][layer] with an 80-byte pitch
   __shared__ __align__(16) unsigned char tile[IT_TOK * 80];
   const long long tt = blockIdx.x;
@@ -725,11 +726,11 @@ __global__ void __launch_bounds__(256) int_transpose_kernel(const CT* __restrict
       uint32_t w[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
       for (int k = 0; k < 4; k++) {
-        uint32_t lo = w[k] & 0xFFFFu, hi = w[k] >> 16;
-        // as signed 16-bit: negative or >= K -> K
-        lo = (!live || lo >= (uint32_t)K) ? (uint32_t)K : lo;
-        hi = (!live || hi >= (uint32_t)K) ? (uint32_t)K : hi;
-        w[k] = lo | (hi << 16);
+        int lo = (short)(w[k] & 0xFFFFu), hi = (short)(w[k] >> 16);
+        if (wrap_negative) { lo += lo < 0 ? K : 0; hi += hi < 0 ? K : 0; }
+        lo = (!live || lo < 0 || lo >= K) ? K : lo;
+        hi = (!live || hi < 0 || hi >= K) ? K : hi;
+        w[k] = (uint32_t)lo | ((uint32_t)hi << 16);
       }
       *reinterpret_cast<uint4*>(tile + i * 80 + c * 16) = make_uint4(w[0], w[1], w[2], w[3]);
     }
@@ -738,7 +739,8 @@ __global__ void __launch_bounds__(256) int_transpose_kernel(const CT* __restrict
       const int i = idx >> 5, j = idx & 31;
       unsigned short v = (unsigned short)K;
       if (t0 + i < T && l0 + j < L) {
-        const long long c = (long long)codes[(t0 + i) * stride + l0 + j];
+        long long c = (long long)codes[(t0 + i) * stride + l0 + j];
+        if (wrap_negative && c < 0) c += K;
         if (c >= 0 && c < K) v = (unsigned short)c;
       }
       *reinterpret_cast<unsigned short*>(tile + i * 80 + j * 2) = v;

@@ -1123,9 +1123,9 @@ static int intensity_impl(const float* cb_norm, int K, const void* codes, int co
   if (!reuse_codes) {
     dim3 grid((unsigned)(L.T_pad / rq::IT_TOK), (unsigned)((L.L + 31) / 32)), block(256);
     uint32_t* ct = (uint32_t*)(ws + L.off_codes);
-    if (code_dtype == 2) rq::int_transpose_kernel<long long><<<grid, block, 0, st>>>((const long long*)codes, code_stride, n_tokens, L.L, K, ct);
-    else if (code_dtype == 1) rq::int_transpose_kernel<int><<<grid, block, 0, st>>>((const int*)codes, code_stride, n_tokens, L.L, K, ct);
-    else rq::int_transpose_kernel<short><<<grid, block, 0, st>>>((const short*)codes, code_stride, n_tokens, L.L, K, ct);
+    if (code_dtype == 2) rq::int_transpose_kernel<long long><<<grid, block, 0, st>>>((const long long*)codes, code_stride, n_tokens, L.L, K, false, ct);
+    else if (code_dtype == 1) rq::int_transpose_kernel<int><<<grid, block, 0, st>>>((const int*)codes, code_stride, n_tokens, L.L, K, false, ct);
+    else rq::int_transpose_kernel<short><<<grid, block, 0, st>>>((const short*)codes, code_stride, n_tokens, L.L, K, false, ct);
     RQ_CUDA(cudaGetLastError());
   }
   // 3. feature operand tiles
@@ -1510,9 +1510,9 @@ int rqae_decode_tc_f32(const float* w_out, const float* b_out, const float* code
   {
     dim3 grid((unsigned)(L.T_pad / rq::IT_TOK), (unsigned)((nq_codes + 31) / 32)), block(256);
     uint32_t* ct = (uint32_t*)(ws + L.off_codes);
-    if (code_dtype == 2) rq::int_transpose_kernel<long long><<<grid, block, 0, st>>>((const long long*)codes, code_stride, n_tokens, nq_codes, K, ct);
-    else if (code_dtype == 1) rq::int_transpose_kernel<int><<<grid, block, 0, st>>>((const int*)codes, code_stride, n_tokens, nq_codes, K, ct);
-    else rq::int_transpose_kernel<short><<<grid, block, 0, st>>>((const short*)codes, code_stride, n_tokens, nq_codes, K, ct);
+    if (code_dtype == 2) rq::int_transpose_kernel<long long><<<grid, block, 0, st>>>((const long long*)codes, code_stride, n_tokens, nq_codes, K, true, ct);
+    else if (code_dtype == 1) rq::int_transpose_kernel<int><<<grid, block, 0, st>>>((const int*)codes, code_stride, n_tokens, nq_codes, K, true, ct);
+    else rq::int_transpose_kernel<short><<<grid, block, 0, st>>>((const short*)codes, code_stride, n_tokens, nq_codes, K, true, ct);
     RQ_CUDA(cudaGetLastError());
   }
   {

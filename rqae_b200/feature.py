@@ -14,6 +14,7 @@ There is no CPU path: code tensors must live on the GPU next to the model.
 """
 from __future__ import annotations
 
+import weakref
 from typing import List, Optional, Sequence
 
 import numpy as np
@@ -62,13 +63,17 @@ def _cuts(layers: Sequence[int]):
 
 class IntensityWorkspace:
     """Caller-owned scratch of ``intensity_many``.  It keeps the tile-major copy of the code tensor between calls: a later
-    call with the same code tensor (same storage, shape and version), the same cuts and codebook size only rebuilds the
-    feature operand (``rqae_intensity_again_f16``) -- scripts/3_make_rqae_features.py:164-196 mines its features group by
-    group over one code store."""
+    call only rebuilds the feature operand (``rqae_intensity_again_f16``) when it passes the very tensor object of the
+    previous call (held by a weak reference), unchanged since (same ``_version``, shape, strides and dtype), with the same
+    cuts and codebook size, and ``intensity_many`` used that tensor as it is (int16 / int32 / int64 with rows of unit
+    stride: no conversion, no ``.contiguous()`` copy).  A new tensor that happens to sit at a freed one's address, or a
+    temporary copy of a tensor that was changed in place, never matches -- scripts/3_make_rqae_features.py:164-196 mines
+    its features group by group over one code store."""
 
     def __init__(self):
         self.buf: Optional[torch.Tensor] = None
         self.key = None
+        self.src: Optional[weakref.ref] = None   # the caller's code tensor behind ``key``
 
 
 def intensity_many(rqae, token_indices: torch.Tensor, centers: torch.Tensor, layers: Sequence[int],
@@ -116,9 +121,12 @@ def intensity_many(rqae, token_indices: torch.Tensor, centers: torch.Tensor, lay
         nbytes = lib.rqae_intensity_workspace_bytes(cuts_arr.ctypes.data, len(cuts), Fn, T)
         if nbytes == 0:
             raise NotImplementedError("unsupported intensity shape (at most 64 distinct cuts / 256 K-blocks)")
-        key = (codes.data_ptr(), codes._version, tuple(codes.shape), codes.stride(0), codes.dtype, tuple(cuts), K, str(dev))
-        again = workspace is not None and workspace.key == key and workspace.buf is not None \
-            and workspace.buf.numel() >= nbytes + 1024
+        # a copy made above is a new tensor on every call: its address and version say nothing about its contents
+        own = codes.untyped_storage().data_ptr() == token_indices.untyped_storage().data_ptr()
+        key = (codes.data_ptr(), token_indices._version, tuple(token_indices.shape), token_indices.stride(), codes.dtype,
+               tuple(cuts), K, str(dev))
+        again = own and workspace is not None and workspace.key == key and workspace.src is not None \
+            and workspace.src() is token_indices and workspace.buf is not None and workspace.buf.numel() >= nbytes + 1024
         if workspace is None:
             ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
         else:
@@ -141,7 +149,7 @@ def intensity_many(rqae, token_indices: torch.Tensor, centers: torch.Tensor, lay
                     cuts_arr.ctypes.data, len(cuts), out.data_ptr(), out.shape[2], ws_ptr, ws_bytes, st)
         _lib.check(rc, "rqae_intensity_again_f16" if again else "rqae_intensity_f16")
         if workspace is not None:
-            workspace.key = key
+            workspace.key, workspace.src = (key, weakref.ref(token_indices)) if own else (None, None)
         for t in (ws, cb_norm, w, centers, codes):
             t.record_stream(torch.cuda.current_stream(dev))
     res = out[:, :, :T]
