@@ -13,21 +13,72 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # RQAE_B200_LIB points the binding at another build of the same library (A/B timing of kernel variants)
 LIB_PATH = os.environ.get("RQAE_B200_LIB") or os.path.join(_HERE, "librqae_b200.so")
 
-# every symbol include/rqae_b200.h declares (tests/test_capi_symbols.py checks the list against the header)
-SYMBOLS = [
-    "rqae_version", "rqae_strerror", "rqae_last_cuda_error", "rqae_packed_bytes", "rqae_pack_weights",
-    "rqae_forward_f32", "rqae_forward_variant", "rqae_hook_rmsnorm", "rqae_decode_f32", "rqae_forward_host_f32", "rqae_forward_host_config", "rqae_forward_host_mode", "rqae_widen_codes_host", "rqae_forward_host_release",
-    "rqae_fp32_peak_probe", "rqae_intensity_again_f16", "rqae_search_tc_store_bytes", "rqae_search_tc_pack_store",
-    "rqae_search_tc_workspace_bytes", "rqae_search_tc_maxima_f16", "rqae_search_rows_f16", "rqae_search_qrows_bytes",
-    "rqae_search_build_qrows_f16",
-    "rqae_launch_count", "rqae_intensity_workspace_bytes", "rqae_intensity_f16",
-    "rqae_select_top_middle_bottom_f16", "rqae_decode_tc_workspace_bytes", "rqae_decode_tc_f32",
-    "rqae_search_table_bytes", "rqae_search_build_table_f16", "rqae_search_accumulate_f16", "rqae_search_position_max_f16",
-]
+_s, _vp, _i, _i64, _sz, _f = (ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_size_t,
+                               ctypes.c_float)
+_pi, _pd = ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_double)
 
-CODE_DTYPE = {"int16": 0, "int32": 1, "int64": 2}
+# name -> (restype, argtypes) of every function include/rqae_b200.h declares, in its order
+# (tests/test_capi_symbols.py checks the names and types against the header)
+BINDINGS = {
+    "rqae_version": (_s, []),
+    "rqae_strerror": (_s, [_i]),
+    "rqae_last_cuda_error": (_s, []),
+    "rqae_packed_bytes": (_sz, [_i, _i, _i, _i]),
+    "rqae_pack_weights": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _sz, _vp]),
+    "rqae_forward_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp, _i, _i64, _vp, _vp, _vp, _vp]),
+    "rqae_forward_variant": (_i, [_i]),
+    "rqae_hook_rmsnorm": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i, _i64, _i, _vp, _f, _i, _i, _vp, _i, _i64, _vp]),
+    "rqae_decode_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _i, _i64, _vp, _vp, _i64, _vp, _vp]),
+    "rqae_forward_host_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp, _i, _vp, _i64]),
+    "rqae_forward_host_config": (_i, [_i, _i]),
+    "rqae_forward_host_mode": (_i, [_pi, _pi]),
+    "rqae_widen_codes_host": (_i, [_vp, _vp, _i64, _i, _i]),
+    "rqae_forward_host_release": (_i, []),
+    "rqae_intensity_workspace_bytes": (_sz, [_vp, _i, _i, _i64]),
+    "rqae_intensity_f16": (_i, [_vp, _i, _vp, _i, _i64, _i64, _vp, _i64, _i, _vp, _vp, _i, _vp, _i64, _vp, _sz, _vp]),
+    "rqae_intensity_again_f16": (_i, [_vp, _i, _i64, _vp, _i64, _i, _vp, _vp, _i, _vp, _i64, _vp, _sz, _vp]),
+    "rqae_select_top_middle_bottom_f16": (_i, [_vp, _i64, _i64, _i64, _i, _vp, _vp, _vp]),
+    "rqae_search_table_bytes": (_sz, [_i, _i]),
+    "rqae_search_build_table_f16": (_i, [_vp, _i, _vp, _i64, _i, _i, _vp, _sz, _vp]),
+    "rqae_search_accumulate_f16": (_i, [_vp, _i, _vp, _i, _i64, _i64, _i, _i, _i, _vp, _vp]),
+    "rqae_search_position_max_f16": (_i, [_vp, _i64, _i, _i, _vp, _i64, _vp]),
+    "rqae_decode_tc_workspace_bytes": (_sz, [_i, _i, _i64, _i]),
+    "rqae_decode_tc_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _i, _i64, _vp, _i64, _vp, _i, _vp, _sz, _vp]),
+    "rqae_fp32_peak_probe": (_i, [_i, _i, _pd, _vp, _vp]),
+    "rqae_search_tc_store_bytes": (_sz, [_i64, _i]),
+    "rqae_search_qrows_bytes": (_sz, [_i, _i, _i]),
+    "rqae_search_build_qrows_f16": (_i, [_vp, _i, _vp, _i64, _i, _i, _vp, _sz, _vp]),
+    "rqae_search_tc_pack_store": (_i, [_vp, _i, _i64, _i64, _i, _i, _i, _vp, _sz, _vp]),
+    "rqae_search_tc_workspace_bytes": (_sz, [_vp, _i]),
+    "rqae_search_tc_maxima_f16": (_i, [_vp, _i64, _i, _i, _vp, _vp, _i, _i, _vp, _i64, _i, _vp, _i, _vp, _i64, _vp, _sz, _vp]),
+    "rqae_search_rows_f16": (_i, [_vp, _i, _vp, _i, _i64, _i64, _i, _vp, _i, _i, _vp, _i, _i, _vp, _vp]),
+    "rqae_launch_count": (_i64, [_i]),
+}
+SYMBOLS = list(BINDINGS)
+
+CODE_DTYPE = {"int16": 0, "int32": 1, "int64": 2}   # the C ABI's code_dtype by dtype name
 
 _lib = None
+
+
+def code_dtype(dtype):
+    """The C ABI's ``code_dtype`` for a torch dtype: 0 int16, 1 int32, 2 int64, None for any other dtype."""
+    return CODE_DTYPE.get(str(dtype).split(".")[-1])
+
+
+def code_tensor(t):
+    """A code tensor in a dtype the C ABI takes: ``t`` itself when it is int16 / int32 / int64, else ``t`` as int64."""
+    return t if code_dtype(t.dtype) is not None else t.long()
+
+
+def workspace(nbytes: int, device, buf=None):
+    """Device scratch of ``nbytes`` bytes at the 1024-byte alignment the tensor-core entry points require: (tensor,
+    aligned pointer, usable bytes from that pointer).  ``buf`` is reused when it is on ``device`` and large enough."""
+    import torch
+    if buf is None or buf.device != device or buf.numel() < nbytes + 1024:
+        buf = torch.empty(nbytes + 1024, dtype=torch.uint8, device=device)
+    ptr = (buf.data_ptr() + 1023) // 1024 * 1024
+    return buf, ptr, buf.numel() - (ptr - buf.data_ptr())
 
 
 def build_hint() -> str:
@@ -42,72 +93,9 @@ def load() -> ctypes.CDLL:
     if not os.path.exists(LIB_PATH):
         raise ImportError(build_hint())
     lib = ctypes.CDLL(LIB_PATH)
-    c = ctypes
-    vp, i, i64, sz = c.c_void_p, c.c_int, c.c_int64, c.c_size_t
-    lib.rqae_version.restype = c.c_char_p
-    lib.rqae_strerror.restype = c.c_char_p
-    lib.rqae_strerror.argtypes = [i]
-    lib.rqae_last_cuda_error.restype = c.c_char_p
-    lib.rqae_packed_bytes.restype = sz
-    lib.rqae_packed_bytes.argtypes = [i, i, i, i]
-    lib.rqae_pack_weights.restype = i
-    lib.rqae_pack_weights.argtypes = [vp, vp, vp, vp, vp, i, i, i, i, i, vp, sz, vp]
-    lib.rqae_forward_f32.restype = i
-    lib.rqae_forward_f32.argtypes = [vp, vp, i, i, i, i, i, i, vp, i64, vp, i, i64, vp, vp, vp, vp]
-    lib.rqae_forward_variant.restype = i
-    lib.rqae_forward_variant.argtypes = [i]
-    lib.rqae_hook_rmsnorm.restype = i
-    lib.rqae_hook_rmsnorm.argtypes = [vp, vp, i, i, i, i, i, i, vp, i, i64, i, vp, c.c_float, i, i, vp, i, i64, vp]
-    lib.rqae_decode_f32.restype = i
-    lib.rqae_decode_f32.argtypes = [vp, vp, i, i, i, i, i, vp, i, i64, vp, vp, i64, vp, vp]
-    lib.rqae_forward_host_f32.restype = i
-    lib.rqae_forward_host_f32.argtypes = [vp, vp, i, i, i, i, i, i, vp, i64, vp, i, vp, i64]
-    lib.rqae_forward_host_config.restype = i
-    lib.rqae_forward_host_config.argtypes = [i, i]
-    lib.rqae_forward_host_mode.restype = i
-    lib.rqae_forward_host_mode.argtypes = [c.POINTER(c.c_int), c.POINTER(c.c_int)]
-    lib.rqae_widen_codes_host.restype = i
-    lib.rqae_widen_codes_host.argtypes = [vp, vp, i64, i, i]
-    lib.rqae_forward_host_release.restype = i
-    lib.rqae_forward_host_release.argtypes = []
-    lib.rqae_fp32_peak_probe.restype = i
-    lib.rqae_fp32_peak_probe.argtypes = [i, i, c.POINTER(c.c_double), vp, vp]
-    lib.rqae_intensity_workspace_bytes.restype = sz
-    lib.rqae_intensity_workspace_bytes.argtypes = [vp, i, i, i64]
-    lib.rqae_intensity_f16.restype = i
-    lib.rqae_intensity_f16.argtypes = [vp, i, vp, i, i64, i64, vp, i64, i, vp, vp, i, vp, i64, vp, sz, vp]
-    lib.rqae_intensity_again_f16.restype = i
-    lib.rqae_intensity_again_f16.argtypes = [vp, i, i64, vp, i64, i, vp, vp, i, vp, i64, vp, sz, vp]
-    lib.rqae_select_top_middle_bottom_f16.restype = i
-    lib.rqae_select_top_middle_bottom_f16.argtypes = [vp, i64, i64, i64, i, vp, vp, vp]
-    lib.rqae_decode_tc_workspace_bytes.restype = sz
-    lib.rqae_decode_tc_workspace_bytes.argtypes = [i, i, i64, i]
-    lib.rqae_decode_tc_f32.restype = i
-    lib.rqae_decode_tc_f32.argtypes = [vp, vp, vp, i, i, i, i, i, vp, i, i64, vp, i64, vp, i, vp, sz, vp]
-    lib.rqae_search_table_bytes.restype = sz
-    lib.rqae_search_table_bytes.argtypes = [i, i]
-    lib.rqae_search_build_table_f16.restype = i
-    lib.rqae_search_build_table_f16.argtypes = [vp, i, vp, i64, i, i, vp, sz, vp]
-    lib.rqae_search_accumulate_f16.restype = i
-    lib.rqae_search_accumulate_f16.argtypes = [vp, i, vp, i, i64, i64, i, i, i, vp, vp]
-    lib.rqae_search_position_max_f16.restype = i
-    lib.rqae_search_position_max_f16.argtypes = [vp, i64, i, i, vp, i64, vp]
-    lib.rqae_search_tc_store_bytes.restype = sz
-    lib.rqae_search_tc_store_bytes.argtypes = [i64, i]
-    lib.rqae_search_tc_pack_store.restype = i
-    lib.rqae_search_tc_pack_store.argtypes = [vp, i, i64, i64, i, i, i, vp, sz, vp]
-    lib.rqae_search_tc_workspace_bytes.restype = sz
-    lib.rqae_search_tc_workspace_bytes.argtypes = [vp, i]
-    lib.rqae_search_tc_maxima_f16.restype = i
-    lib.rqae_search_tc_maxima_f16.argtypes = [vp, i64, i, i, vp, vp, i, i, vp, i64, i, vp, i, vp, i64, vp, sz, vp]
-    lib.rqae_search_qrows_bytes.restype = sz
-    lib.rqae_search_qrows_bytes.argtypes = [i, i, i]
-    lib.rqae_search_build_qrows_f16.restype = i
-    lib.rqae_search_build_qrows_f16.argtypes = [vp, i, vp, i64, i, i, vp, sz, vp]
-    lib.rqae_search_rows_f16.restype = i
-    lib.rqae_search_rows_f16.argtypes = [vp, i, vp, i, i64, i64, i, vp, i, i, vp, i, i, vp, vp]
-    lib.rqae_launch_count.restype = i64
-    lib.rqae_launch_count.argtypes = [i]
+    for name, (restype, argtypes) in BINDINGS.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = lib
     return lib
 

@@ -12,6 +12,7 @@
 #include <map>
 #include <mutex>
 #include <thread>
+#include <tuple>
 #include <vector>
 #include <math.h>
 #if defined(__x86_64__) && !defined(RQ_NO_STREAM)
@@ -51,20 +52,33 @@ thread_local int64_t g_launches = 0;
     }                                    \
   } while (0)
 
-// Opt a kernel in to its dynamic shared-memory size, once per (kernel, device): the attribute is per device, and a
-// process may drive more than one.
-cudaError_t ensure_dynamic_smem(const void* kern, int bytes) {
+// Counts a kernel launch that the runtime accepted (rqae_launch_count) and returns the launch's error.
+cudaError_t launched(cudaError_t e = cudaGetLastError()) {
+  if (e == cudaSuccess) g_launches++;
+  return e;
+}
+
+// Set a function attribute of a kernel once per (kernel, attribute, device) and remember the result: attributes are
+// per device, and a process may drive more than one.
+cudaError_t ensure_func_attr(const void* kern, cudaFuncAttribute attr, int value) {
   static std::mutex mu;
-  static std::map<std::pair<const void*, int>, cudaError_t> done;
+  static std::map<std::tuple<const void*, int, int>, cudaError_t> done;
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return e;
   std::lock_guard<std::mutex> lock(mu);
-  auto it = done.find({kern, dev});
+  const auto key = std::make_tuple(kern, (int)attr, dev);
+  auto it = done.find(key);
   if (it != done.end()) return it->second;
-  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  done[{kern, dev}] = e;
-  return e;
+  return done[key] = cudaFuncSetAttribute(kern, attr, value);
+}
+
+// Calls f with a value of the C++ type of code_dtype (RQAE_CODE_*): the kernels that read codes are templates on it.
+template <typename F>
+void with_code_type(int code_dtype, F&& f) {
+  if (code_dtype == RQAE_CODE_I64) f((long long)0);
+  else if (code_dtype == RQAE_CODE_I32) f((int)0);
+  else f((short)0);
 }
 
 // A stream-ordered pool of this library's own per device, for the few bytes per row of the selection's fallback list.
@@ -372,29 +386,34 @@ __global__ void __launch_bounds__(256, 1) fma_pattern_probe_kernel(int iters, fl
 // ---------------------------------------------------------------------------------------------
 // forward launch
 // ---------------------------------------------------------------------------------------------
+// Takes the next of the forward kernel's lock-step counters (one per launch in flight) and zeroes it on `st`.
+cudaError_t lockstep_slot(cudaStream_t st, unsigned int** slot) {
+  unsigned int* base = nullptr;
+  cudaError_t e = cudaGetSymbolAddress((void**)&base, g_sync_ctr);
+  if (e != cudaSuccess) return e;
+  *slot = base + (g_launch_seq.fetch_add(1) % kSyncSlots) * 32;
+  return cudaMemsetAsync(*slot, 0, sizeof(unsigned int), st);
+}
+
 template <int E, int EC, int CH, int NSLOT, int TG, bool DBG, bool HOOK = false>
 int launch_forward_t(const rq::FwdParams& prm, int sms, cudaStream_t st) {
   using C = rq::FwdCfg<E, EC, CH, NSLOT, TG>;
   auto kern = rq::rq_forward_kernel<E, EC, CH, NSLOT, TG, DBG, HOOK>;
-  RQ_CUDA(ensure_dynamic_smem((const void*)kern, C::SM_TOTAL));
+  RQ_CUDA(ensure_func_attr((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SM_TOTAL));
   const long long n_units = (prm.n_tokens + 2 * TG - 1) / (2 * TG);
   const int grid = (int)(n_units < sms ? n_units : sms);
   rq::FwdParams p2 = prm;
   p2.sync_ctr = nullptr;
   if (n_units > grid) {
-    // more than one unit per CTA: keep the CTAs' weight streams in step (one counter per launch in flight).
+    // more than one unit per CTA: keep the CTAs' weight streams in step.
     // The kernel spins on the counter, so all CTAs must be co-resident: cooperative launch guarantees it.
-    unsigned int* base = nullptr;
-    RQ_CUDA(cudaGetSymbolAddress((void**)&base, g_sync_ctr));
-    p2.sync_ctr = base + (g_launch_seq.fetch_add(1) % kSyncSlots) * 32;
-    RQ_CUDA(cudaMemsetAsync(p2.sync_ctr, 0, sizeof(unsigned int), st));
+    RQ_CUDA(lockstep_slot(st, &p2.sync_ctr));
     void* args[] = {(void*)&p2};
-    RQ_CUDA(cudaLaunchCooperativeKernel((const void*)kern, dim3(grid), dim3(rq::kThreads), args, C::SM_TOTAL, st));
+    RQ_CUDA(launched(cudaLaunchCooperativeKernel((const void*)kern, dim3(grid), dim3(rq::kThreads), args, C::SM_TOTAL, st)));
   } else {
     kern<<<grid, rq::kThreads, C::SM_TOTAL, st>>>(p2);
-    RQ_CUDA(cudaGetLastError());
+    RQ_CUDA(launched());
   }
-  g_launches++;
   return RQAE_OK;
 }
 
@@ -404,7 +423,7 @@ template <int E, int EC, int CH, int NSLOT, int TG, bool DBG, int CS>
 int launch_forward_cluster_t(const rq::FwdParams& prm, int sms, cudaStream_t st) {
   using C = rq::FwdCfg<E, EC, CH, NSLOT, TG, CS>;
   auto kern = rq::rq_forward_kernel<E, EC, CH, NSLOT, TG, DBG, false, CS>;
-  RQ_CUDA(ensure_dynamic_smem((const void*)kern, C::SM_TOTAL));
+  RQ_CUDA(ensure_func_attr((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SM_TOTAL));
   static std::mutex mu;
   static std::map<int, int> max_clusters;   // per device
   int dev = 0;
@@ -439,16 +458,10 @@ int launch_forward_cluster_t(const rq::FwdParams& prm, int sms, cudaStream_t st)
   rq::FwdParams p2 = prm;
   p2.sync_ctr = nullptr;
   const bool coop = n_units > clusters;
-  if (coop) {
-    unsigned int* base = nullptr;
-    RQ_CUDA(cudaGetSymbolAddress((void**)&base, g_sync_ctr));
-    p2.sync_ctr = base + (g_launch_seq.fetch_add(1) % kSyncSlots) * 32;
-    RQ_CUDA(cudaMemsetAsync(p2.sync_ctr, 0, sizeof(unsigned int), st));
-  }
+  if (coop) RQ_CUDA(lockstep_slot(st, &p2.sync_ctr));
   cfg.gridDim = dim3((unsigned)(clusters * CS));
   cfg.numAttrs = coop ? 2 : 1;
-  RQ_CUDA(cudaLaunchKernelEx(&cfg, kern, p2));
-  g_launches++;
+  RQ_CUDA(launched(cudaLaunchKernelEx(&cfg, kern, p2)));
   return RQAE_OK;
 }
 
@@ -463,6 +476,53 @@ int launch_forward(const rq::FwdParams& prm, int sms, cudaStream_t st) {
   if (prm.hs != nullptr) return launch_forward_t<E, EC, CH, NSLOT, TG, false, true>(prm, sms, st);
   if (prm.teacher != nullptr || prm.z_out != nullptr) return launch_forward_t<E, EC, CH, NSLOT, TG, true>(prm, sms, st);
   return launch_forward_t<E, EC, CH, NSLOT, TG, false>(prm, sms, st);
+}
+
+// ---------------------------------------------------------------------------------------------
+// tcgen05 GEMM of the intensities, the tensor-core decode and the tensor-core search maxima (rq_intensity.cuh)
+// ---------------------------------------------------------------------------------------------
+// Workspace of the intensity and tensor-core decode GEMMs: schedule, weight prefixes, fp16 lookup tables, the decode's
+// bias, layer-major int16 codes of L layers, feature operand tiles; every segment rounded up to 1 KB.  The codes come
+// before the feature tiles so that their place does not depend on F: rqae_intensity_again_f16 reuses them.
+struct GemmLayout {
+  int L, NKB, F_tiles;
+  long long T_pad;
+  size_t off_sched, off_wcum, off_lut, off_bias, off_codes, off_u, total;
+  long long units() const { return (T_pad / rq::IT_TOK) * (long long)((F_tiles + 1) / 2); }
+};
+
+GemmLayout gemm_layout(int L, int nkb, int F, int64_t n_tokens, bool bias) {
+  GemmLayout o;
+  o.L = L;
+  o.NKB = nkb;
+  o.F_tiles = (F + rq::IT_FT - 1) / rq::IT_FT;
+  o.T_pad = (n_tokens + rq::IT_TOK - 1) / rq::IT_TOK * rq::IT_TOK;
+  auto up = [](size_t v) { return (v + 1023) / 1024 * 1024; };
+  size_t off = 0;
+  o.off_sched = off; off = up(off + (size_t)rq::IT_MAX_KB * sizeof(rq::IntKBlock));
+  o.off_wcum = off;  off = up(off + 2 * (size_t)rq::IT_MAX_CUTS * 4);
+  o.off_lut = off;   off = up(off + 2 * (size_t)rq::IT_LUT_ROWS * 8);
+  o.off_bias = off;  off = up(off + (bias ? (size_t)o.F_tiles * rq::IT_FT * 4 : 0));
+  o.off_codes = off; off = up(off + (size_t)L * (size_t)o.T_pad * 2);
+  o.off_u = off;     off = up(off + (size_t)o.F_tiles * nkb * rq::IT_U_TILE);
+  o.total = off;
+  return o;
+}
+
+// Runs the GEMM on min(units, sms) persistent CTAs.  Only the intensity epilogue stores through a tensor map; the
+// others are given a zeroed one.
+template <int EPI>
+int launch_gemm(const rq::IntParams& ip, long long units, int sms, const CUtensorMap* out_map, cudaStream_t st) {
+  constexpr int smem = rq::IntSmemOf<EPI>::type::TOTAL;
+  auto kern = rq::rq_intensity_kernel<EPI>;
+  RQ_CUDA(ensure_func_attr((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  CUtensorMap map;
+  if (out_map) map = *out_map;
+  else memset(&map, 0, sizeof(map));
+  const int grid = (int)(units < sms ? units : sms);
+  kern<<<grid, rq::IT_THREADS, smem, st>>>(ip, map);
+  RQ_CUDA(launched());
+  return RQAE_OK;
 }
 
 }  // namespace
@@ -514,14 +574,12 @@ int rqae_pack_weights(const float* w_in, const float* b_in, const float* w_out, 
   const long long total = (long long)(nq + 1) * s.E * RQ_GROUP_THREADS;
   pack_stages_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w_in, b_in, w_out, b_out, nq, dim, s.E, s.CH, pk,
                                                                       L.off_bin, L.off_stage, L.stage_bytes);
-  g_launches++;
-  RQ_CUDA(cudaGetLastError());
+  RQ_CUDA(launched());
   if (L.off_stage_cl) {   // second copy for the D-split cluster variant: one chunk per CTA of the cluster
     pack_stages_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w_in, b_in, w_out, b_out, nq, dim, s.E,
                                                                         rq_cluster_size(s.E), pk, L.off_bin, L.off_stage_cl,
                                                                         L.stage_bytes);
-    g_launches++;
-    RQ_CUDA(cudaGetLastError());
+    RQ_CUDA(launched());
   }
   if (codebook_shared) {
     // the table is tiny: fetch it, build the search tables on the host, upload (this entry point therefore
@@ -667,16 +725,14 @@ int rqae_fp32_peak_probe(int packed_f32x2, int iters, double* flops_per_launch, 
   if (packed_f32x2 >= 2) {   // operand-pattern probes (see fma_pattern_probe_kernel); sink doubles as the data source
     if (packed_f32x2 == 2) fma_pattern_probe_kernel<2><<<sms, 256, 0, (cudaStream_t)stream>>>(iters, sink, sink + 64);
     else fma_pattern_probe_kernel<3><<<sms, 256, 0, (cudaStream_t)stream>>>(iters, sink, sink + 64);
-    g_launches++;
-    RQ_CUDA(cudaGetLastError());
+    RQ_CUDA(launched());
     if (flops_per_launch) *flops_per_launch = (double)sms * 256 * (double)iters * (packed_f32x2 == 2 ? 48.0 : 60.0) * 4.0;
     return RQAE_OK;
   }
   const int grid = sms * 2, block = 512;
   if (packed_f32x2) fp32_probe_kernel<true><<<grid, block, 0, (cudaStream_t)stream>>>(iters, sink);
   else fp32_probe_kernel<false><<<grid, block, 0, (cudaStream_t)stream>>>(iters, sink);
-  g_launches++;
-  RQ_CUDA(cudaGetLastError());
+  RQ_CUDA(launched());
   if (flops_per_launch) *flops_per_launch = (double)grid * block * (double)iters * 8.0 * 24.0 * 2.0;
   return RQAE_OK;
 }
@@ -1031,43 +1087,23 @@ static int make_out_map(void* out, int64_t out_stride, int n_cuts, int n_feature
   return RQAE_OK;
 }
 
-struct IntLayout {
-  int L, NKB, F_tiles;
-  long long T_pad;
-  size_t off_sched, off_wcum, off_lut, off_u, off_codes, total;
-};
-
-struct IntLayout;
-static long long ip_units(const IntLayout& L);
-static int int_layout(const int32_t* cuts, int n_cuts, int F, int64_t n_tokens, int nq, IntLayout* o) {
+// The intensity workspace for a list of cuts (strictly ascending layer indices).
+static int int_layout(const int32_t* cuts, int n_cuts, int F, int64_t n_tokens, GemmLayout* o) {
   if (!cuts || n_cuts <= 0 || n_cuts > rq::IT_MAX_CUTS || F <= 0 || n_tokens < 0) return RQAE_EINVAL;
   int prev = -1, nkb = 0;
   for (int c = 0; c < n_cuts; c++) {
-    if (cuts[c] <= prev || (nq > 0 && cuts[c] >= nq)) return RQAE_EINVAL;   // strictly ascending layer indices
+    if (cuts[c] <= prev) return RQAE_EINVAL;   // strictly ascending layer indices
     nkb += (cuts[c] - prev + rq::IT_LPB - 1) / rq::IT_LPB;
     prev = cuts[c];
   }
   if (nkb > rq::IT_MAX_KB) return RQAE_EUNSUPPORTED;
-  o->L = prev + 1;
-  o->NKB = nkb;
-  o->F_tiles = (F + rq::IT_FT - 1) / rq::IT_FT;
-  o->T_pad = (n_tokens + rq::IT_TOK - 1) / rq::IT_TOK * rq::IT_TOK;
-  auto up = [](size_t v) { return (v + 1023) / 1024 * 1024; };
-  size_t off = 0;
-  o->off_sched = off; off = up(off + (size_t)rq::IT_MAX_KB * sizeof(rq::IntKBlock));
-  o->off_wcum = off;  off = up(off + 2 * (size_t)rq::IT_MAX_CUTS * 4);
-  o->off_lut = off;   off = up(off + 2 * (size_t)rq::IT_LUT_ROWS * 8);
-  o->off_codes = off; off = up(off + (size_t)o->L * (size_t)o->T_pad * 2);   // before the feature tiles: its place does not depend on F
-  o->off_u = off;     off = up(off + (size_t)o->F_tiles * nkb * rq::IT_U_TILE);
-  o->total = off;
+  *o = gemm_layout(prev + 1, nkb, F, n_tokens, false);
   return RQAE_OK;
 }
 
-static long long ip_units(const IntLayout& L) { return (L.T_pad / rq::IT_TOK) * (long long)((L.F_tiles + 1) / 2); }
-
 size_t rqae_intensity_workspace_bytes(const int32_t* cuts_host, int n_cuts, int n_features, int64_t n_tokens) {
-  IntLayout L;
-  if (int_layout(cuts_host, n_cuts, n_features, n_tokens, 0, &L)) return 0;
+  GemmLayout L;
+  if (int_layout(cuts_host, n_cuts, n_features, n_tokens, &L)) return 0;
   return L.total;
 }
 
@@ -1099,8 +1135,8 @@ static int intensity_impl(const float* cb_norm, int K, const void* codes, int co
   if (!cb_norm || (!codes && !reuse_codes) || !centers || !layer_weights_f16 || !out || !workspace || K <= 0) return RQAE_EINVAL;
   if (code_dtype < 0 || code_dtype > 2) return RQAE_EINVAL;
   if (K + 1 > rq::IT_LUT_ROWS) return RQAE_EUNSUPPORTED;
-  IntLayout L;
-  int rc = int_layout(cuts_host, n_cuts, n_features, n_tokens, 0, &L);
+  GemmLayout L;
+  int rc = int_layout(cuts_host, n_cuts, n_features, n_tokens, &L);
   if (rc) return rc;
   if (code_stride < L.L || center_stride < L.L) return RQAE_EINVAL;
   if (out_stride < L.T_pad || (out_stride & 7) || ((uintptr_t)out & 15)) return RQAE_EINVAL;   // 16-byte row stores of 256 tokens
@@ -1118,15 +1154,16 @@ static int intensity_impl(const float* cb_norm, int K, const void* codes, int co
   pp.n_cuts = n_cuts; pp.K = K; pp.cb_norm = cb_norm; pp.w = (const __half*)layer_weights_f16;
   pp.sched = (rq::IntKBlock*)(ws + L.off_sched); pp.wcum = (float*)(ws + L.off_wcum); pp.lut = (uint2*)(ws + L.off_lut);
   rq::int_prep_kernel<<<4, 256, 0, st>>>(pp);
-  RQ_CUDA(cudaGetLastError());
+  RQ_CUDA(launched());
   // 2. codes -> layer-major int16 (kept from the previous call on this workspace when the caller says they are the same)
   if (!reuse_codes) {
     dim3 grid((unsigned)(L.T_pad / rq::IT_TOK), (unsigned)((L.L + 31) / 32)), block(256);
     uint32_t* ct = (uint32_t*)(ws + L.off_codes);
-    if (code_dtype == 2) rq::int_transpose_kernel<long long><<<grid, block, 0, st>>>((const long long*)codes, code_stride, n_tokens, L.L, K, false, ct);
-    else if (code_dtype == 1) rq::int_transpose_kernel<int><<<grid, block, 0, st>>>((const int*)codes, code_stride, n_tokens, L.L, K, false, ct);
-    else rq::int_transpose_kernel<short><<<grid, block, 0, st>>>((const short*)codes, code_stride, n_tokens, L.L, K, false, ct);
-    RQ_CUDA(cudaGetLastError());
+    with_code_type(code_dtype, [&](auto tag) {
+      using CT = decltype(tag);
+      rq::int_transpose_kernel<CT><<<grid, block, 0, st>>>((const CT*)codes, code_stride, n_tokens, L.L, K, false, ct);
+    });
+    RQ_CUDA(launched());
   }
   // 3. feature operand tiles
   {
@@ -1134,27 +1171,21 @@ static int intensity_impl(const float* cb_norm, int K, const void* codes, int co
     rq::int_pack_u_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(
         centers, center_stride, n_features, L.F_tiles, L.NKB, (const rq::IntKBlock*)(ws + L.off_sched), cb_norm, K,
         (const __half*)layer_weights_f16, ws + L.off_u);
-    RQ_CUDA(cudaGetLastError());
+    RQ_CUDA(launched());
   }
   // 4. the GEMM
-  RQ_CUDA(ensure_dynamic_smem((const void*)rq::rq_intensity_kernel<0>, rq::IntSmem::TOTAL));
   rq::IntParams ip;
   ip.codes_p = (const uint32_t*)(ws + L.off_codes); ip.L = L.L; ip.T_pad = L.T_pad; ip.u_tiles = ws + L.off_u;
   ip.sched = (const rq::IntKBlock*)(ws + L.off_sched); ip.wcum = (const float*)(ws + L.off_wcum);
   ip.lut = (const uint2*)(ws + L.off_lut); ip.K = K; ip.NKB = L.NKB; ip.n_cuts = n_cuts; ip.F = n_features;
-  const long long units = ip_units(L);
   // start groups 20 k clocks apart when every CTA has several units to run
-  ip.stagger = units >= 4LL * sms && n_cuts >= 4 ? 20000 : 0;
+  ip.stagger = L.units() >= 4LL * sms && n_cuts >= 4 ? 20000 : 0;
   ip.q_out = nullptr; ip.bias = nullptr; ip.T = n_tokens; ip.D = 0;
   ip.F_tiles = L.F_tiles; ip.out = (__half*)out; ip.out_stride = out_stride; ip.n_tok_tiles = L.T_pad / rq::IT_TOK;
-  const int grid = (int)(units < sms ? units : sms);
   CUtensorMap out_map;
   rc = make_out_map(out, out_stride, n_cuts, n_features, &out_map);
   if (rc) return rc;
-  rq::rq_intensity_kernel<0><<<grid, rq::IT_THREADS, rq::IntSmem::TOTAL, st>>>(ip, out_map);
-  RQ_CUDA(cudaGetLastError());
-  g_launches += reuse_codes ? 3 : 4;
-  return RQAE_OK;
+  return launch_gemm<0>(ip, L.units(), sms, &out_map, st);
 }
 
 int rqae_select_top_middle_bottom_f16(const void* vals, int64_t rows, int64_t row_stride, int64_t n, int top_k,
@@ -1197,31 +1228,29 @@ int rqae_select_top_middle_bottom_f16(const void* vals, int64_t rows, int64_t ro
       mp.fb_count = fb; mp.fb_list = fb + 1;
       constexpr int smem3 = (int)sizeof(rq::Mine3Smem);
       static_assert(2 * (smem3 + 1024) <= 227 * 1024, "two CTAs per SM");
-      e = ensure_dynamic_smem((const void*)rq::rq_mine3_kernel, smem3);
+      e = ensure_func_attr((const void*)rq::rq_mine3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem3);
       if (e == cudaSuccess) {
         const int grid = (int)(rows < 2LL * sms ? rows : 2LL * sms);
         rq::rq_mine3_kernel<<<grid, rq::M3_THREADS, smem3, st>>>(mp);
-        e = cudaGetLastError();
+        e = launched();
       }
-      if (e == cudaSuccess) e = ensure_dynamic_smem((const void*)rq::rq_mine2_kernel, smem2);
+      if (e == cudaSuccess) e = ensure_func_attr((const void*)rq::rq_mine2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2);
       if (e == cudaSuccess) {
         rq::MineParams fp = mp;
         fp.row_count = fb; fp.row_list = fb + 1;
         const long long cap = (long long)sms * per_sm2;
         rq::rq_mine2_kernel<<<(int)(rows < cap ? rows : cap), rq::M2_THREADS, smem2, st>>>(fp);
-        e = cudaGetLastError();
+        e = launched();
       }
     }
     cudaFreeAsync(fb, st);
     RQ_CUDA(e);
-    g_launches += 2;
     return RQAE_OK;
   }
-  RQ_CUDA(ensure_dynamic_smem((const void*)rq::rq_mine2_kernel, smem2));
+  RQ_CUDA(ensure_func_attr((const void*)rq::rq_mine2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
   const int grid = (int)(rows < (long long)sms * per_sm2 ? rows : (long long)sms * per_sm2);
   rq::rq_mine2_kernel<<<grid, rq::M2_THREADS, smem2, st>>>(mp);
-  RQ_CUDA(cudaGetLastError());
-  g_launches++;
+  RQ_CUDA(launched());
   return RQAE_OK;
 }
 
@@ -1247,8 +1276,7 @@ int rqae_search_build_table_f16(const void* sims_f16, int K, const int32_t* quer
   tp.n_query = n_query; tp.n_layers = n_layers; tp.K = K; tp.table = (__half*)table;
   dim3 grid((unsigned)((K + 31) / 32), (unsigned)n_layers);
   rq::search_table_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(tp);
-  RQ_CUDA(cudaGetLastError());
-  g_launches++;
+  RQ_CUDA(launched());
   return RQAE_OK;
 }
 
@@ -1267,12 +1295,10 @@ int rqae_search_accumulate_f16(const void* table, int K, const void* codes, int 
   ap.K = K; ap.layer_begin = layer_begin; ap.layer_end = layer_end; ap.first = first ? 1 : 0; ap.acc = (__half*)acc;
   const long long tiles = (n_tokens + rq::SR_TILE - 1) / rq::SR_TILE;
   const int grid = (int)(tiles < 4LL * sms ? tiles : 4LL * sms);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (code_dtype == RQAE_CODE_I64) rq::search_accumulate_kernel<long long><<<grid, rq::SR_THREADS, 0, st>>>(ap);
-  else if (code_dtype == RQAE_CODE_I32) rq::search_accumulate_kernel<int><<<grid, rq::SR_THREADS, 0, st>>>(ap);
-  else rq::search_accumulate_kernel<short><<<grid, rq::SR_THREADS, 0, st>>>(ap);
-  RQ_CUDA(cudaGetLastError());
-  g_launches++;
+  with_code_type(code_dtype, [&](auto tag) {
+    rq::search_accumulate_kernel<decltype(tag)><<<grid, rq::SR_THREADS, 0, (cudaStream_t)stream>>>(ap);
+  });
+  RQ_CUDA(launched());
   return RQAE_OK;
 }
 
@@ -1292,8 +1318,7 @@ int rqae_search_position_max_f16(const void* acc, int64_t n_seq, int seq_len, in
   const long long blocks = (out_stride + 31) / 32;
   if (blocks >= (1LL << 31)) return RQAE_EUNSUPPORTED;
   rq::search_posmax_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(mp);
-  RQ_CUDA(cudaGetLastError());
-  g_launches++;
+  RQ_CUDA(launched());
   return RQAE_OK;
 }
 
@@ -1330,12 +1355,12 @@ int rqae_search_tc_pack_store(const void* codes, int code_dtype, int64_t code_st
   if (units >= (1LL << 31)) return RQAE_EUNSUPPORTED;
   const int L8 = (nq_codes + 7) / 8;
   dim3 grid((unsigned)units, (unsigned)(L8 < 8 ? L8 : 8));
-  cudaStream_t st = (cudaStream_t)stream;
-  if (code_dtype == RQAE_CODE_I64) rq::srch_pack_store_kernel<long long><<<grid, 256, 0, st>>>((const long long*)codes, code_stride, n_seq, seq_len, nq_codes, K, L8, (uint4*)store_tc);
-  else if (code_dtype == RQAE_CODE_I32) rq::srch_pack_store_kernel<int><<<grid, 256, 0, st>>>((const int*)codes, code_stride, n_seq, seq_len, nq_codes, K, L8, (uint4*)store_tc);
-  else rq::srch_pack_store_kernel<short><<<grid, 256, 0, st>>>((const short*)codes, code_stride, n_seq, seq_len, nq_codes, K, L8, (uint4*)store_tc);
-  RQ_CUDA(cudaGetLastError());
-  g_launches++;
+  with_code_type(code_dtype, [&](auto tag) {
+    using CT = decltype(tag);
+    rq::srch_pack_store_kernel<CT><<<grid, 256, 0, (cudaStream_t)stream>>>((const CT*)codes, code_stride, n_seq, seq_len,
+                                                                          nq_codes, K, L8, (uint4*)store_tc);
+  });
+  RQ_CUDA(launched());
   return RQAE_OK;
 }
 
@@ -1371,37 +1396,22 @@ int rqae_search_tc_maxima_f16(const void* store_tc, int64_t n_seq, int seq_len, 
   for (int c = 0; c < n_layers_list; c++) pp.ends[c] = layers_host[c];
   pp.n_cuts = n_layers_list; pp.sched = (rq::IntKBlock*)ws;
   rq::srch_prep_kernel<<<1, 32, 0, st>>>(pp);
-  RQ_CUDA(cudaGetLastError());
+  RQ_CUDA(launched());
   {
     const int total = nkb * rq::IT_FT * 8;
     rq::srch_pack_u_kernel<<<(total + 255) / 256, 256, 0, st>>>(query, query_stride, n_query, last, K, (const uint4*)utab_f16,
                                                                (const rq::IntKBlock*)ws, nkb, ws + 4096);
-    RQ_CUDA(cudaGetLastError());
+    RQ_CUDA(launched());
   }
-  RQ_CUDA(ensure_dynamic_smem((const void*)rq::rq_intensity_kernel<2>, rq::IntSmemS::TOTAL));
-  {   // leave the rest of the SM's 256 KB to L1: the factor gathers re-use sectors within a K-block
-    static std::mutex mu;
-    static std::map<int, cudaError_t> done;
-    int dev = 0;
-    RQ_CUDA(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(mu);
-    if (!done.count(dev))
-      done[dev] = cudaFuncSetAttribute((const void*)rq::rq_intensity_kernel<2>, cudaFuncAttributePreferredSharedMemoryCarveout, 58);
-    RQ_CUDA(done[dev]);
-  }
+  // leave the rest of the SM's 256 KB to L1: the factor gathers re-use sectors within a K-block
+  RQ_CUDA(ensure_func_attr((const void*)rq::rq_intensity_kernel<2>, cudaFuncAttributePreferredSharedMemoryCarveout, 58));
   rq::IntParams ip;
   memset(&ip, 0, sizeof(ip));
   ip.u_tiles = ws + 4096; ip.sched = (const rq::IntKBlock*)ws; ip.K = K; ip.NKB = nkb; ip.n_cuts = n_layers_list;
   ip.F = n_query; ip.F_tiles = 1; ip.n_tok_tiles = units; ip.L = last; ip.T_pad = units * rq::IT_TOK;
   ip.s_codes = (const uint4*)store_tc; ip.s_vtab = (const uint4*)vtab_f16; ip.s_max = (__half*)max_out;
   ip.s_stride = max_stride; ip.s_len = seq_len; ip.L8 = L8; ip.stagger = 0;
-  const int grid = (int)(units < sms ? units : sms);
-  CUtensorMap no_map;
-  memset(&no_map, 0, sizeof(no_map));
-  rq::rq_intensity_kernel<2><<<grid, rq::IT_THREADS, rq::IntSmemS::TOTAL, st>>>(ip, no_map);
-  RQ_CUDA(cudaGetLastError());
-  g_launches += 3;
-  return RQAE_OK;
+  return launch_gemm<2>(ip, units, sms, nullptr, st);
 }
 
 size_t rqae_search_qrows_bytes(int n_layers, int n_query, int K) {
@@ -1417,8 +1427,7 @@ int rqae_search_build_qrows_f16(const void* sims_f16, int K, const int32_t* quer
   dim3 grid((unsigned)n_query, (unsigned)n_layers);
   rq::search_qrows_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((const __half*)sims_f16, query, query_stride, n_query, n_layers, K,
                                                                   (__half*)qrows);
-  RQ_CUDA(cudaGetLastError());
-  g_launches++;
+  RQ_CUDA(launched());
   return RQAE_OK;
 }
 
@@ -1442,44 +1451,26 @@ int rqae_search_rows_f16(const void* table, int K, const void* codes, int code_d
   rp.out = (__half*)rows_out;
   if (K > rq::SRW_KMAX || n_seq * (int64_t)seq_len >= 0xFFFFFFFFLL) return RQAE_EUNSUPPORTED;
   const unsigned blocks = (unsigned)(n_query * n_cuts);                      // one block per (cut, query position)
-  cudaStream_t st = (cudaStream_t)stream;
-  if (code_dtype == RQAE_CODE_I64) rq::search_rows_kernel<long long><<<blocks, rq::SRW_THREADS, 0, st>>>(rp);
-  else if (code_dtype == RQAE_CODE_I32) rq::search_rows_kernel<int><<<blocks, rq::SRW_THREADS, 0, st>>>(rp);
-  else rq::search_rows_kernel<short><<<blocks, rq::SRW_THREADS, 0, st>>>(rp);
-  RQ_CUDA(cudaGetLastError());
-  g_launches++;
+  with_code_type(code_dtype, [&](auto tag) {
+    rq::search_rows_kernel<decltype(tag)><<<blocks, rq::SRW_THREADS, 0, (cudaStream_t)stream>>>(rp);
+  });
+  RQ_CUDA(launched());
   return RQAE_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
 // tensor-core decode (opt-in; rq_decode.cuh is the bit-exact default)
 // ---------------------------------------------------------------------------------------------
-struct DecTcLayout {
-  int NKB, F_tiles;
-  long long T_pad;
-  size_t off_sched, off_wcum, off_lut, off_bias, off_u, off_codes, total;
-};
-
-static int dec_tc_layout(int nq_codes, int dim, int64_t n_tokens, int passes, DecTcLayout* o) {
+static int dec_tc_layout(int nq_codes, int dim, int64_t n_tokens, int passes, GemmLayout* o) {
   if (nq_codes <= 0 || dim <= 0 || n_tokens < 0 || (passes != 1 && passes != 3)) return RQAE_EINVAL;
-  o->NKB = passes * ((nq_codes + rq::IT_LPB - 1) / rq::IT_LPB);
-  if (o->NKB > rq::IT_MAX_KB) return RQAE_EUNSUPPORTED;
-  o->F_tiles = (dim + rq::IT_FT - 1) / rq::IT_FT;
-  o->T_pad = (n_tokens + rq::IT_TOK - 1) / rq::IT_TOK * rq::IT_TOK;
-  auto up = [](size_t v) { return (v + 1023) / 1024 * 1024; };
-  size_t off = 0;
-  o->off_sched = off; off = up(off + (size_t)rq::IT_MAX_KB * sizeof(rq::IntKBlock));
-  o->off_wcum = off;  off = up(off + 2 * (size_t)rq::IT_MAX_CUTS * 4);
-  o->off_lut = off;   off = up(off + 2 * (size_t)rq::IT_LUT_ROWS * 8);
-  o->off_bias = off;  off = up(off + (size_t)o->F_tiles * rq::IT_FT * 4);
-  o->off_u = off;     off = up(off + (size_t)o->F_tiles * o->NKB * rq::IT_U_TILE);
-  o->off_codes = off; off = up(off + (size_t)nq_codes * (size_t)o->T_pad * 2);
-  o->total = off;
+  const int nkb = passes * ((nq_codes + rq::IT_LPB - 1) / rq::IT_LPB);
+  if (nkb > rq::IT_MAX_KB) return RQAE_EUNSUPPORTED;
+  *o = gemm_layout(nq_codes, nkb, dim, n_tokens, true);
   return RQAE_OK;
 }
 
 size_t rqae_decode_tc_workspace_bytes(int nq_codes, int dim, int64_t n_tokens, int passes) {
-  DecTcLayout L;
+  GemmLayout L;
   if (dec_tc_layout(nq_codes, dim, n_tokens, passes, &L)) return 0;
   return L.total;
 }
@@ -1492,7 +1483,7 @@ int rqae_decode_tc_f32(const float* w_out, const float* b_out, const float* code
     return RQAE_EINVAL;
   if (code_dtype < 0 || code_dtype > 2 || code_stride < nq_codes) return RQAE_EINVAL;
   if (codebook_dim != 4 || K + 1 > rq::IT_LUT_ROWS) return RQAE_EUNSUPPORTED;
-  DecTcLayout L;
+  GemmLayout L;
   int rc = dec_tc_layout(nq_codes, dim, n_tokens, passes, &L);
   if (rc) return rc;
   if (((uintptr_t)workspace & 1023) || workspace_bytes < L.total) return RQAE_ESIZE;
@@ -1506,25 +1497,25 @@ int rqae_decode_tc_f32(const float* w_out, const float* b_out, const float* code
   pp.L = nq_codes; pp.K = K; pp.passes = passes; pp.codebook0 = codebook0;
   pp.sched = (rq::IntKBlock*)(ws + L.off_sched); pp.wcum = (float*)(ws + L.off_wcum); pp.lut = (uint2*)(ws + L.off_lut);
   rq::dec_prep_kernel<<<4, 256, 0, st>>>(pp);
-  RQ_CUDA(cudaGetLastError());
+  RQ_CUDA(launched());
   {
     dim3 grid((unsigned)(L.T_pad / rq::IT_TOK), (unsigned)((nq_codes + 31) / 32)), block(256);
     uint32_t* ct = (uint32_t*)(ws + L.off_codes);
-    if (code_dtype == 2) rq::int_transpose_kernel<long long><<<grid, block, 0, st>>>((const long long*)codes, code_stride, n_tokens, nq_codes, K, true, ct);
-    else if (code_dtype == 1) rq::int_transpose_kernel<int><<<grid, block, 0, st>>>((const int*)codes, code_stride, n_tokens, nq_codes, K, true, ct);
-    else rq::int_transpose_kernel<short><<<grid, block, 0, st>>>((const short*)codes, code_stride, n_tokens, nq_codes, K, true, ct);
-    RQ_CUDA(cudaGetLastError());
+    with_code_type(code_dtype, [&](auto tag) {
+      using CT = decltype(tag);
+      rq::int_transpose_kernel<CT><<<grid, block, 0, st>>>((const CT*)codes, code_stride, n_tokens, nq_codes, K, true, ct);
+    });
+    RQ_CUDA(launched());
   }
   {
     const long long total = (long long)L.F_tiles * L.NKB * rq::IT_FT * rq::IT_LPB;
     rq::dec_pack_u_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w_out, dim, L.F_tiles, L.NKB,
                                                                           (const rq::IntKBlock*)(ws + L.off_sched), layer_mask,
                                                                           ws + L.off_u);
-    RQ_CUDA(cudaGetLastError());
+    RQ_CUDA(launched());
     rq::dec_bias_kernel<<<(dim + 127) / 128, 128, 0, st>>>(b_out, nq_codes, dim, layer_mask, (float*)(ws + L.off_bias));
-    RQ_CUDA(cudaGetLastError());
+    RQ_CUDA(launched());
   }
-  RQ_CUDA(ensure_dynamic_smem((const void*)rq::rq_intensity_kernel<1>, rq::IntSmem::TOTAL));
   rq::IntParams ip;
   memset(&ip, 0, sizeof(ip));
   ip.codes_p = (const uint32_t*)(ws + L.off_codes); ip.L = nq_codes; ip.T_pad = L.T_pad; ip.u_tiles = ws + L.off_u;
@@ -1532,14 +1523,7 @@ int rqae_decode_tc_f32(const float* w_out, const float* b_out, const float* code
   ip.lut = (const uint2*)(ws + L.off_lut); ip.K = K; ip.NKB = L.NKB; ip.n_cuts = 1; ip.F = dim; ip.F_tiles = L.F_tiles;
   ip.n_tok_tiles = L.T_pad / rq::IT_TOK; ip.q_out = q_out; ip.bias = (const float*)(ws + L.off_bias); ip.T = n_tokens; ip.D = dim;
   ip.stagger = 0;
-  const long long units = ip.n_tok_tiles * ((L.F_tiles + 1) / 2);
-  const int grid = (int)(units < sms ? units : sms);
-  CUtensorMap no_map;
-  memset(&no_map, 0, sizeof(no_map));   // the decode epilogue stores with plain instructions
-  rq::rq_intensity_kernel<1><<<grid, rq::IT_THREADS, rq::IntSmem::TOTAL, st>>>(ip, no_map);
-  RQ_CUDA(cudaGetLastError());
-  g_launches += 5;
-  return RQAE_OK;
+  return launch_gemm<1>(ip, L.units(), sms, nullptr, st);   // the decode epilogue stores with plain instructions
 }
 
 }  // extern "C"

@@ -91,9 +91,7 @@ def intensity_many(rqae, token_indices: torch.Tensor, centers: torch.Tensor, lay
         raise RuntimeError("rqae_b200 intensity needs the code tensor on the GPU; there is no CPU fallback")
     dev = token_indices.device
     lib = _lib.load()
-    codes = token_indices
-    if codes.dtype not in (torch.int16, torch.int32, torch.int64):
-        codes = codes.to(torch.int64)
+    codes = _lib.code_tensor(token_indices)
     nq_codes = codes.shape[-1]
     codes = codes.reshape(-1, nq_codes)
     if codes.stride(-1) != 1 or (codes.shape[0] > 1 and codes.stride(0) < nq_codes):
@@ -125,18 +123,12 @@ def intensity_many(rqae, token_indices: torch.Tensor, centers: torch.Tensor, lay
         own = codes.untyped_storage().data_ptr() == token_indices.untyped_storage().data_ptr()
         key = (codes.data_ptr(), token_indices._version, tuple(token_indices.shape), token_indices.stride(), codes.dtype,
                tuple(cuts), K, str(dev))
+        ws, ws_ptr, ws_bytes = _lib.workspace(nbytes, dev, None if workspace is None else workspace.buf)
+        # the codes of the previous call are still in the workspace only if it kept its buffer
         again = own and workspace is not None and workspace.key == key and workspace.src is not None \
-            and workspace.src() is token_indices and workspace.buf is not None and workspace.buf.numel() >= nbytes + 1024
-        if workspace is None:
-            ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
-        else:
-            if not again:
-                if workspace.buf is None or workspace.buf.numel() < nbytes + 1024 or workspace.buf.device != dev:
-                    workspace.buf = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
-                workspace.key = None          # set below, once the codes are in place
-            ws = workspace.buf
-        ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
-        ws_bytes = ws.numel() - (ws_ptr - ws.data_ptr())
+            and workspace.src() is token_indices and ws is workspace.buf
+        if workspace is not None and not again:
+            workspace.buf, workspace.key = ws, None   # key set below, once the codes are in place
         with torch.cuda.device(dev):
             st = torch.cuda.current_stream(dev).cuda_stream
             if again:
@@ -144,7 +136,7 @@ def intensity_many(rqae, token_indices: torch.Tensor, centers: torch.Tensor, lay
                                                   cuts_arr.ctypes.data, len(cuts), out.data_ptr(), out.shape[2], ws_ptr, ws_bytes, st)
             else:
                 rc = lib.rqae_intensity_f16(
-                    cb_norm.data_ptr(), K, codes.data_ptr(), _lib.CODE_DTYPE[str(codes.dtype).split(".")[-1]],
+                    cb_norm.data_ptr(), K, codes.data_ptr(), _lib.code_dtype(codes.dtype),
                     codes.stride(0) if T > 1 else nq_codes, T, centers.data_ptr(), centers.shape[1], Fn, w.data_ptr(),
                     cuts_arr.ctypes.data, len(cuts), out.data_ptr(), out.shape[2], ws_ptr, ws_bytes, st)
         _lib.check(rc, "rqae_intensity_again_f16" if again else "rqae_intensity_f16")

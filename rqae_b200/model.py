@@ -253,7 +253,7 @@ class RQAE(nn.Module):
                 rc = lib.rqae_forward_f32(
                     packed.data_ptr(), cb_arg.data_ptr(), int(shared), self.num_quantizers, nq_run, self.dim,
                     self.codebook_dim, self.codebook.shape[1], xc.data_ptr(), n, codes.data_ptr(),
-                    _lib.CODE_DTYPE[str(out_dtype).split(".")[-1]], nq_run,
+                    _lib.code_dtype(out_dtype), nq_run,
                     0 if q is None else q.data_ptr(), 0 if tch is None else tch.data_ptr(),
                     0 if z is None else z.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
             _lib.check(rc, "rqae_forward_f32")
@@ -296,11 +296,9 @@ class RQAE(nn.Module):
         lib = _lib.load()
         dev = src.device
         if codes is not None:
-            if codes.dtype not in (torch.int16, torch.int32, torch.int64):
-                codes = codes.to(torch.int64)
-            codes = codes.contiguous()
+            codes = _lib.code_tensor(codes).contiguous()
             lead, nq_codes = codes.shape[:-1], codes.shape[-1]
-            code_dtype = _lib.CODE_DTYPE[str(codes.dtype).split(".")[-1]]
+            code_dtype = _lib.code_dtype(codes.dtype)
         else:
             if cv.shape[-1] != self.codebook_dim:
                 raise RuntimeError("codebook values must have last dimension codebook_dim")
@@ -349,9 +347,7 @@ class RQAE(nn.Module):
             raise RuntimeError("rqae_b200.RQAE.decode needs CUDA tensors; there is no CPU fallback")
         lib = _lib.load()
         dev = codes.device
-        if codes.dtype not in (torch.int16, torch.int32, torch.int64):
-            codes = codes.to(torch.int64)
-        codes = codes.contiguous()
+        codes = _lib.code_tensor(codes).contiguous()
         lead, nq_codes = codes.shape[:-1], min(codes.shape[-1], self.num_quantizers)
         mask, any_sel = self._layer_mask(layers, nq_codes, dev)
         if not any_sel:
@@ -373,14 +369,13 @@ class RQAE(nn.Module):
         nbytes = lib.rqae_decode_tc_workspace_bytes(nq_codes, self.dim, n, passes)
         if nbytes == 0:
             raise NotImplementedError("tensor-core decode supports at most 3200 layer-passes (nq * passes)")
-        ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
-        ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
+        ws, ws_ptr, ws_bytes = _lib.workspace(nbytes, dev)
         with torch.cuda.device(dev):
             rc = lib.rqae_decode_tc_f32(
                 w_out.data_ptr(), b_out.data_ptr(), cb0.data_ptr(), self.num_quantizers, nq_codes, self.dim,
-                self.codebook_dim, self.codebook.shape[1], codes.data_ptr(),
-                _lib.CODE_DTYPE[str(codes.dtype).split(".")[-1]], codes.shape[-1], 0 if mask is None else mask.data_ptr(),
-                n, q.data_ptr(), passes, ws_ptr, nbytes, torch.cuda.current_stream(dev).cuda_stream)
+                self.codebook_dim, self.codebook.shape[1], codes.data_ptr(), _lib.code_dtype(codes.dtype),
+                codes.shape[-1], 0 if mask is None else mask.data_ptr(), n, q.data_ptr(), passes, ws_ptr, ws_bytes,
+                torch.cuda.current_stream(dev).cuda_stream)
         _lib.check(rc, "rqae_decode_tc_f32")
         for t in (ws, cb0, codes):
             t.record_stream(torch.cuda.current_stream(dev))
@@ -436,7 +431,7 @@ class RQAE(nn.Module):
                 rc = _lib.load().rqae_forward_host_f32(
                     packed.data_ptr(), cb_arg.data_ptr(), int(shared), self.num_quantizers, nq_run, self.dim,
                     self.codebook_dim, self.codebook.shape[1], xc.data_ptr(), n, codes.data_ptr(),
-                    _lib.CODE_DTYPE[str(out_dtype).split(".")[-1]], 0 if q is None else q.data_ptr(), int(chunk_tokens))
+                    _lib.code_dtype(out_dtype), 0 if q is None else q.data_ptr(), int(chunk_tokens))
             _lib.check(rc, "rqae_forward_host_f32")
         return q, codes
 
@@ -488,7 +483,7 @@ class RQAE(nn.Module):
                     packed.data_ptr(), cb_arg.data_ptr(), int(shared), self.num_quantizers, self.num_quantizers, self.dim,
                     self.codebook_dim, self.codebook.shape[1], hidden.data_ptr(), hd, n, S, w.data_ptr(), float(rms_eps),
                     int(bool(skip_bos)), int(bool(replace)), 0 if codes is None else codes.data_ptr(),
-                    _lib.CODE_DTYPE[str(out_dtype).split(".")[-1]], self.num_quantizers,
+                    _lib.code_dtype(out_dtype), self.num_quantizers,
                     torch.cuda.current_stream(dev).cuda_stream)
             _lib.check(rc, "rqae_hook_rmsnorm")
         return codes

@@ -29,8 +29,6 @@ SQ_PAD = 128          # rq_search.cuh SR_Q: query positions are padded to one 25
 SELECT_KMAX = 256     # rq_mine.cuh MN_KMAX
 SERVER_LAYERS = [4, 6, 8, 12, 16, 24, 32, 48, 64, 128, 256, 512, 1023]   # server.py:167
 
-_CODE_DTYPE = {torch.int16: 0, torch.int32: 1, torch.int64: 2}
-
 
 def engine_sims(model, mode: str = "projected") -> torch.Tensor:
     """server.py:103-115: the (nq, K, K) fp16 table of the engine."""
@@ -108,7 +106,7 @@ class IntensityEngine:
             activations = torch.cat([a.to(self.sims.device) for a in activations], dim=0)
         if not activations.is_cuda:
             raise RuntimeError("IntensityEngine needs the code store on the GPU; there is no CPU fallback")
-        if activations.dim() != 3 or activations.dtype not in _CODE_DTYPE:
+        if activations.dim() != 3 or _lib.code_dtype(activations.dtype) is None:
             raise ValueError("activations must be an int16/int32/int64 tensor (sequences, positions, num_quantizers)")
         if activations.shape[0] == 0 or activations.shape[1] == 0:
             raise ValueError("the code store is empty")
@@ -135,7 +133,7 @@ class IntensityEngine:
         nbytes = lib.rqae_search_tc_store_bytes(N, nq_codes)
         self._store_tc = torch.empty(nbytes // 2, dtype=torch.int16, device=dev)
         with torch.cuda.device(dev):
-            _lib.check(lib.rqae_search_tc_pack_store(self.activations.data_ptr(), _CODE_DTYPE[self.activations.dtype], nq_codes,
+            _lib.check(lib.rqae_search_tc_pack_store(self.activations.data_ptr(), _lib.code_dtype(self.activations.dtype), nq_codes,
                                                     N, S, nq_codes, K, self._store_tc.data_ptr(), nbytes,
                                                     torch.cuda.current_stream(dev).cuda_stream), "rqae_search_tc_pack_store")
 
@@ -159,8 +157,7 @@ class IntensityEngine:
         wbytes = lib.rqae_search_tc_workspace_bytes(lh.data_ptr(), len(layers))
         if wbytes == 0:
             raise NotImplementedError("precision='tc': too many layer ranges for one launch")
-        ws = torch.empty(wbytes + 1024, dtype=torch.uint8, device=dev)
-        off = (-ws.data_ptr()) % 1024
+        ws, ws_ptr, ws_bytes = _lib.workspace(wbytes, dev)
         stride = ((N + 1) // 2 * 2 + 7) // 8 * 8
         out = torch.empty(len(layers), SQ_PAD, stride, dtype=torch.float16, device=dev)
         if stride > (N + 1) // 2 * 2:     # the kernel writes two columns per unit; the selection's 16-byte loads touch the padding
@@ -170,7 +167,7 @@ class IntensityEngine:
             _lib.check(lib.rqae_search_tc_maxima_f16(self._store_tc.data_ptr(), N, S, nq_codes, self._vtab.data_ptr(),
                                                     self._utab.data_ptr(), self._vtab.shape[0], K, query.data_ptr(),
                                                     query.stride(0), Sq, lh.data_ptr(), len(layers), out.data_ptr(), stride,
-                                                    ws.data_ptr() + off, wbytes, st), "rqae_search_tc_maxima_f16")
+                                                    ws_ptr, ws_bytes, st), "rqae_search_tc_maxima_f16")
         ws.record_stream(torch.cuda.current_stream(dev))
         return out[:, :, :N] if padded else out[:, :Sq, :N]     # padded: all 128 rows per cut (rows >= Sq are zero)
 
@@ -192,7 +189,7 @@ class IntensityEngine:
         lh = torch.tensor([int(l) for l in layers], dtype=torch.int32)
         with torch.cuda.device(dev):
             _lib.check(_lib.load().rqae_search_rows_f16(table.data_ptr(), K, self.activations.data_ptr(),
-                                                       _CODE_DTYPE[self.activations.dtype], nq_codes, N, S, sel.data_ptr(), Sq,
+                                                       _lib.code_dtype(self.activations.dtype), nq_codes, N, S, sel.data_ptr(), Sq,
                                                        n_sel, lh.data_ptr(), int(first_range), C, out.data_ptr(),
                                                        torch.cuda.current_stream(dev).cuda_stream), "rqae_search_rows_f16")
         return out[0] if single else out
@@ -284,7 +281,7 @@ class IntensityEngine:
                     last = cur
                 st = cur.cuda_stream
                 _lib.check(lib.rqae_search_accumulate_f16(table.data_ptr(), K, self.activations.data_ptr(),
-                                                         _CODE_DTYPE[self.activations.dtype], nq_codes, N * S, a, b,
+                                                         _lib.code_dtype(self.activations.dtype), nq_codes, N * S, a, b,
                                                          1 if a == 0 else 0, acc.data_ptr(), st), "rqae_search_accumulate_f16")
                 _lib.check(lib.rqae_search_position_max_f16(acc.data_ptr(), N, S, Sq, maxv.data_ptr(), n_pad, st),
                            "rqae_search_position_max_f16")

@@ -18,6 +18,35 @@ def test_header_and_binding_list_agree():
     assert header_symbols() == sorted(_lib.SYMBOLS)
 
 
+def header_prototypes():
+    """name -> (return type, [parameter types]) of every function include/rqae_b200.h declares, as C text."""
+    src = open(os.path.join(ROOT, "include", "rqae_b200.h")).read()
+    src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
+    protos = {}
+    for ret, name, params in re.findall(r"([\w ]+\*?)\s*\b(rqae_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", src):
+        params = [] if params.strip() == "void" else [re.sub(r"\s*\w+$", "", p.strip()) for p in params.split(",")]
+        protos[name] = (" ".join(ret.split()), [" ".join(p.split()) for p in params])
+    return protos
+
+
+def test_binding_types_match_the_header():
+    c = ctypes
+    known = {"int": c.c_int, "int64_t": c.c_int64, "size_t": c.c_size_t, "float": c.c_float, "const char*": c.c_char_p,
+             "int*": c.POINTER(c.c_int), "double*": c.POINTER(c.c_double)}   # int* / double*: out-parameters
+
+    def ctype(decl):   # any other pointer is a data pointer
+        return known.get(decl, c.c_void_p if decl.endswith("*") else None)
+
+    protos = header_prototypes()
+    assert sorted(protos) == header_symbols()
+    for name, (ret, params) in protos.items():
+        restype, argtypes = _lib.BINDINGS[name]
+        assert restype is ctype(ret), f"{name}: returns {ret}, bound as {restype}"
+        assert len(argtypes) == len(params), f"{name}: {len(params)} parameters, {len(argtypes)} bound"
+        for k, (decl, bound) in enumerate(zip(params, argtypes)):
+            assert bound is ctype(decl), f"{name}: parameter {k} is {decl}, bound as {bound}"
+
+
 def test_library_exports_every_declared_symbol():
     lib = ctypes.CDLL(_lib.LIB_PATH)
     for name in header_symbols():
