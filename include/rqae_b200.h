@@ -178,6 +178,28 @@ int rqae_intensity_again_f16(const float* cb_norm, int K, int64_t n_tokens, cons
                              int n_features, const void* layer_weights_f16, const int32_t* cuts_host, int n_cuts, void* out,
                              int64_t out_stride, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Bit-exact RQAEFeature.intensity (rqae/feature.py:102-129) for `n_features` features at once: the reference's own
+ * arithmetic, rounding for rounding (the opt-in exact path; rqae_intensity_f16 is the faster tolerance path).  For
+ * feature f, token t and every cut (cuts_host: strictly ascending layer indices, deepest <= 4095, any number):
+ *     p_l  = fp16( w_l * sims[centers[f][l]][codes[t][l]] )                    one rounding
+ *     run  = +0.0f; run += float(p_l), l = 0, 1, ...       wrun likewise of float(w_l), both fp32, ascending layers
+ *     out[f][c][t] = fp16( float(fp16(run)) / float(fp16(wrun)) )              IEEE fp32 divide
+ * Code indexing is the reference's sims[center, codes]: a token or center code in [-K, 0) reads row code + K; a code
+ * outside [-K, K), where the reference raises, contributes a +0 product.  (rqae_intensity_f16 treats every code
+ * outside [0, K) as 0.)
+ *   sims_f16           fp16 [K][K], the reference's codebook_sims (rqae/model.py:140-142), K < 640
+ *   codes              [n_tokens][code_stride] of code_dtype, code_stride > deepest cut
+ *   centers            int32 [n_features][center_stride], center_stride > deepest cut
+ *   layer_weights_f16  fp16 [>= deepest cut + 1]; the weight prefixes are summed on the device
+ *   out                fp16 [n_features][n_cuts][out_stride], out_stride >= n_tokens rounded up to 8 and a multiple
+ *                      of 8, 16-byte aligned: the layout rqae_select_top_middle_bottom_f16 reads.  Only tokens
+ *                      < n_tokens are written.
+ * No workspace.  One launch on `stream` (none when n_tokens or n_features is 0); no synchronisation. */
+int rqae_intensity_exact_f16(const void* sims_f16, int K, const void* codes, int code_dtype, int64_t code_stride,
+                             int64_t n_tokens, const int32_t* centers, int64_t center_stride, int n_features,
+                             const void* layer_weights_f16, const int32_t* cuts_host, int n_cuts, void* out,
+                             int64_t out_stride, void* stream);
+
 /* The selection step of the mining loop, scripts/3_make_rqae_features.py:116-128: for every row
  * (one feature at one cut) of `vals`, the positions of the top_k largest values, of the 2*(top_k/2)
  * values around the median rank and of the top_k smallest, i.e. argsort(descending)[:k],

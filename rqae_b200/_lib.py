@@ -37,6 +37,7 @@ BINDINGS = {
     "rqae_intensity_workspace_bytes": (_sz, [_vp, _i, _i, _i64]),
     "rqae_intensity_f16": (_i, [_vp, _i, _vp, _i, _i64, _i64, _vp, _i64, _i, _vp, _vp, _i, _vp, _i64, _vp, _sz, _vp]),
     "rqae_intensity_again_f16": (_i, [_vp, _i, _i64, _vp, _i64, _i, _vp, _vp, _i, _vp, _i64, _vp, _sz, _vp]),
+    "rqae_intensity_exact_f16": (_i, [_vp, _i, _vp, _i, _i64, _i64, _vp, _i64, _i, _vp, _vp, _i, _vp, _i64, _vp]),
     "rqae_select_top_middle_bottom_f16": (_i, [_vp, _i64, _i64, _i64, _i, _vp, _vp, _vp]),
     "rqae_search_table_bytes": (_sz, [_i, _i]),
     "rqae_search_build_table_f16": (_i, [_vp, _i, _vp, _i64, _i, _i, _vp, _sz, _vp]),

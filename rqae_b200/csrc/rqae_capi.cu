@@ -23,6 +23,7 @@
 #include "rq_decode.cuh"
 #include "rq_forward.cuh"
 #include "rq_intensity.cuh"
+#include "rq_intensity_exact.cuh"
 #include "rq_mine.cuh"
 #include "rq_mine3.cuh"
 #include "rq_search.cuh"
@@ -1186,6 +1187,47 @@ static int intensity_impl(const float* cb_norm, int K, const void* codes, int co
   rc = make_out_map(out, out_stride, n_cuts, n_features, &out_map);
   if (rc) return rc;
   return launch_gemm<0>(ip, L.units(), sms, &out_map, st);
+}
+
+int rqae_intensity_exact_f16(const void* sims_f16, int K, const void* codes, int code_dtype, int64_t code_stride,
+                             int64_t n_tokens, const int32_t* centers, int64_t center_stride, int n_features,
+                             const void* layer_weights_f16, const int32_t* cuts_host, int n_cuts, void* out,
+                             int64_t out_stride, void* stream) {
+  if (!sims_f16 || !codes || !centers || !layer_weights_f16 || !cuts_host || !out) return RQAE_EINVAL;
+  if (K <= 0 || code_dtype < 0 || code_dtype > 2 || n_tokens < 0 || n_features < 0 || n_cuts <= 0) return RQAE_EINVAL;
+  if (K >= rq::IX_ROWS) return RQAE_EUNSUPPORTED;   // K + 1 slab rows
+  int prev = -1;
+  for (int c = 0; c < n_cuts; c++) {
+    if (cuts_host[c] <= prev) return RQAE_EINVAL;   // strictly ascending, >= 0
+    prev = cuts_host[c];
+    if (prev >= rq::IX_MAX_LAYERS) return RQAE_EUNSUPPORTED;
+  }
+  if (code_stride <= prev || center_stride <= prev) return RQAE_EINVAL;
+  if (out_stride < (n_tokens + 7) / 8 * 8 || (out_stride & 7) || ((uintptr_t)out & 15)) return RQAE_EINVAL;   // the selection's rows
+  if (n_tokens == 0 || n_features == 0) return RQAE_OK;
+  int sms = 0;
+  int rc = device_sm_count(&sms);
+  if (rc) return rc;
+  rq::IxParams xp;
+  memset(&xp, 0, sizeof(xp));
+  for (int c = 0; c < n_cuts; c++) xp.cut_mask[cuts_host[c] >> 5] |= 1u << (cuts_host[c] & 31);
+  xp.sims = (const __half*)sims_f16; xp.codes = codes; xp.code_stride = code_stride; xp.n_tokens = n_tokens;
+  xp.n_tiles = (n_tokens + rq::IX_TILE - 1) / rq::IX_TILE; xp.centers = centers; xp.center_stride = center_stride;
+  xp.w = (const __half*)layer_weights_f16; xp.out = (__half*)out; xp.out_stride = out_stride;
+  xp.K = K; xp.F = n_features; xp.n_groups = (n_features + rq::IX_FG - 1) / rq::IX_FG; xp.n_cuts = n_cuts; xp.L = prev + 1;
+  const long long units = xp.n_tiles * xp.n_groups;
+  const unsigned grid = (unsigned)std::min<long long>(units, 2LL * sms);   // two CTAs per SM
+  cudaError_t e = cudaSuccess;
+  with_code_type(code_dtype, [&](auto tag) {
+    const void* kern = (const void*)rq::rq_intensity_exact_kernel<decltype(tag)>;
+    e = ensure_func_attr(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, rq::IX_SMEM);
+    if (e == cudaSuccess) {
+      rq::rq_intensity_exact_kernel<decltype(tag)><<<grid, rq::IX_THREADS, rq::IX_SMEM, (cudaStream_t)stream>>>(xp);
+      e = launched();
+    }
+  });
+  RQ_CUDA(e);
+  return RQAE_OK;
 }
 
 int rqae_select_top_middle_bottom_f16(const void* vals, int64_t rows, int64_t row_stride, int64_t n, int top_k,

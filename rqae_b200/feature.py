@@ -8,7 +8,9 @@ and result of ``intensity(token_indices, layers=None) -> (..., len(layers))`` fp
 
 New: ``intensity_many`` evaluates MANY features over a code tensor in one launch sequence -- the inner
 loop of ``scripts/3_make_rqae_features.py:98-114`` (one ``intensity`` call per feature and 1024-sequence
-batch there) -- and returns the feature-major layout the mining step consumes.
+batch there) -- and returns the feature-major layout the mining step consumes.  ``precision="exact"``
+(``rqae_intensity_exact_f16``) reproduces the reference's values bit for bit; the default ``"tc"`` GEMM
+agrees with them within 2e-3.
 
 There is no CPU path: code tensors must live on the GPU next to the model.
 """
@@ -55,6 +57,20 @@ def layer_weights_f16(rqae) -> torch.Tensor:
     return torch.tensor([l[1].weight.data.norm(dim=0).mean().item() for l in rqae.layers]).to(torch.float16)
 
 
+def exact_sims(rqae, device) -> torch.Tensor:
+    """The reference's own ``codebook_sims`` table (model.py:140-142, computed on the host as there) on ``device``, for
+    ``precision="exact"``.  Cached per codebook storage and version; ``RQAE._apply`` drops the cache.  (The model's
+    ``codebook_sims`` property of a CUDA model is a device matmul, which nothing shows to equal the host table.)"""
+    cb = rqae.codebook
+    key = (cb.untyped_storage().data_ptr(), cb._version, str(device))
+    hit = rqae.__dict__.get("_exact_sims")
+    if hit is None or hit[0] != key:
+        n = F.normalize(cb.data.detach()[0].cpu().float(), dim=-1)
+        hit = (key, (n @ n.T).half().to(device))
+        rqae.__dict__["_exact_sims"] = hit
+    return hit[1]
+
+
 def _cuts(layers: Sequence[int]):
     cuts = sorted(set(int(l) for l in layers))
     pos = {l: i for i, l in enumerate(cuts)}
@@ -78,13 +94,21 @@ class IntensityWorkspace:
 
 def intensity_many(rqae, token_indices: torch.Tensor, centers: torch.Tensor, layers: Sequence[int],
                    layer_weights: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None,
-                   workspace: Optional[IntensityWorkspace] = None) -> torch.Tensor:
+                   workspace: Optional[IntensityWorkspace] = None, precision: str = "tc") -> torch.Tensor:
     """Intensities of F features over T tokens at the given layer cuts.
 
     token_indices (..., nq) integer codes on the GPU (int16 / int32 / int64); centers (F, nq) integer;
     returns fp16 (F, len(layers), T) with T = prod(...), feature-major: ``result[f, j]`` is the contiguous
     vector the reference calls ``all_intensities[:, j]`` for feature f (scripts/3:115-119).  ``out`` may be
-    a caller-owned fp16 buffer (F, n_cuts_sorted, >= T rounded up to 256) to reuse between calls."""
+    a caller-owned fp16 buffer (F, n_cuts_sorted, >= T rounded up to 256) to reuse between calls.
+
+    precision="tc" (default): the tcgen05 GEMM, within 2e-3 of the reference, at most 64 distinct cuts.
+    precision="exact": the reference's arithmetic bit for bit (rqae_intensity_exact_f16) for the given fp16 layer
+    weights and codebook[0] -- note that ``layer_weights_f16`` computes the column norms on the model's device; any
+    number of cuts; codes in [-K, 0) index as in the reference; ``out`` needs >= T rounded up to 8 columns; ``workspace``
+    is not used."""
+    if precision not in ("tc", "exact"):
+        raise ValueError(f"unknown intensity precision {precision!r} (expected 'tc' or 'exact')")
     if rqae.quantization_method != "round_fsq":
         raise ValueError("Codebook sims only supported for round_fsq for now")   # model.py:139
     if not token_indices.is_cuda:
@@ -106,16 +130,29 @@ def intensity_many(rqae, token_indices: torch.Tensor, centers: torch.Tensor, lay
     w = w.to(device=dev, dtype=torch.float16).contiguous()
     if w.numel() <= cuts[-1]:
         raise IndexError("layer_weights shorter than the deepest cut")
-    cb_norm = F.normalize(rqae.codebook.data.detach()[0].to(device=dev, dtype=torch.float32), dim=-1).contiguous()
-    K = cb_norm.shape[0]
     cuts_arr = np.asarray(cuts, dtype=np.int32)
-    T_pad = (T + TOKEN_TILE - 1) // TOKEN_TILE * TOKEN_TILE
+    pad = 8 if precision == "exact" else TOKEN_TILE
+    T_pad = (T + pad - 1) // pad * pad
     if out is None:
         out = torch.empty(Fn, len(cuts), T_pad, dtype=torch.float16, device=dev)
     elif out.dtype != torch.float16 or out.device != dev or out.dim() != 3 or out.shape[0] != Fn \
             or out.shape[1] != len(cuts) or out.shape[2] < T_pad or not out.is_contiguous():
-        raise RuntimeError("out must be a contiguous fp16 CUDA tensor (F, unique cuts, >= T rounded up to 256)")
-    if T > 0:
+        raise RuntimeError(f"out must be a contiguous fp16 CUDA tensor (F, unique cuts, >= T rounded up to {pad})")
+    if precision == "exact":
+        if T > 0 and Fn > 0:
+            sims = exact_sims(rqae, dev)
+            with torch.cuda.device(dev):
+                st = torch.cuda.current_stream(dev)
+                rc = lib.rqae_intensity_exact_f16(
+                    sims.data_ptr(), sims.shape[0], codes.data_ptr(), _lib.code_dtype(codes.dtype),
+                    codes.stride(0) if T > 1 else nq_codes, T, centers.data_ptr(), centers.shape[1], Fn, w.data_ptr(),
+                    cuts_arr.ctypes.data, len(cuts), out.data_ptr(), out.shape[2], st.cuda_stream)
+            _lib.check(rc, "rqae_intensity_exact_f16")
+            for t in (sims, w, centers, codes):
+                t.record_stream(st)
+    elif T > 0:
+        cb_norm = F.normalize(rqae.codebook.data.detach()[0].to(device=dev, dtype=torch.float32), dim=-1).contiguous()
+        K = cb_norm.shape[0]
         nbytes = lib.rqae_intensity_workspace_bytes(cuts_arr.ctypes.data, len(cuts), Fn, T)
         if nbytes == 0:
             raise NotImplementedError("unsupported intensity shape (at most 64 distinct cuts / 256 K-blocks)")
@@ -233,13 +270,15 @@ class RQAEFeature:
         self.layer_weights = layer_weights_f16(rqae)
         return self
 
-    def intensity(self, token_indices: torch.Tensor, layers=None):
-        """feature.py:102-129: (..., num_quantizers) codes -> (..., len(layers)) fp16 intensities."""
+    def intensity(self, token_indices: torch.Tensor, layers=None, *, precision: str = "tc"):
+        """feature.py:102-129: (..., num_quantizers) codes -> (..., len(layers)) fp16 intensities.  ``precision="exact"``
+        gives the reference's values bit for bit, for any number of layers (``intensity_many``)."""
         if layers is None:
             layers = self.layers
         if self.rqae is None:
             raise ValueError("Model not loaded. Needed for intensity calculation.")
-        res = intensity_many(self.rqae, token_indices, self.center.reshape(1, -1), layers, layer_weights=self.layer_weights)
+        res = intensity_many(self.rqae, token_indices, self.center.reshape(1, -1), layers, layer_weights=self.layer_weights,
+                             precision=precision)
         return res[0].transpose(0, 1).reshape(*token_indices.shape[:-1], len(layers))
 
     @classmethod
@@ -294,7 +333,8 @@ class FeatureHelper:
     (``{layer: [{"text": ..., "activations": fp16 ndarray (positions,)}, ...]}``, sequences of the top / middle /
     bottom-k tokens in order of first appearance); ``get_activations_many`` does the same for a list of features with
     ONE intensity GEMM and ONE selection launch instead of one container per feature (scripts/3:189-191).  Equal
-    intensities are ordered by token index (the reference's unstable argsort leaves them unspecified)."""
+    intensities are ordered by token index (the reference's unstable argsort leaves them unspecified).  ``precision`` is
+    that of ``intensity_many``: with ``"exact"`` every activation row equals the reference's bit for bit."""
 
     FEATURE_FOLDER = "/data/datasets/monology_pile/features/rqae-rqae-round_fsq-cbd4-cbs5-nq1024"   # scripts/3:152-158
 
@@ -324,7 +364,8 @@ class FeatureHelper:
             return self.texts[index[0].item()]
         return self.texts[index[0].item()][index[1].item()]
 
-    def get_activations_many(self, features: Sequence["RQAEFeature"], layers: list = None, top_k: int = 100) -> List[dict]:
+    def get_activations_many(self, features: Sequence["RQAEFeature"], layers: list = None, top_k: int = 100,
+                             precision: str = "tc") -> List[dict]:
         if not features:
             return []
         if layers is None:
@@ -337,7 +378,7 @@ class FeatureHelper:
         if "_workspace" not in self.__dict__:
             self._workspace = IntensityWorkspace()       # the code store's tile-major copy survives from one feature group to the next
         inten = intensity_many(rqae, self.indices, centers, layers, layer_weights=features[0].layer_weights,
-                               workspace=self._workspace)                                                      # (F, C, T)
+                               workspace=self._workspace, precision=precision)                                 # (F, C, T)
         sel, _ = select_top_middle_bottom(inten, top_k)                                                        # (F, C, 3, k)
         sel = sel.cpu()
         mid = 2 * (top_k // 2)
@@ -352,10 +393,11 @@ class FeatureHelper:
             results.append(activations)
         return results
 
-    def get_activations(self, rqae: "RQAEFeature", layers: list = None, top_k: int = 100, index=None):
+    def get_activations(self, rqae: "RQAEFeature", layers: list = None, top_k: int = 100, index=None,
+                        precision: str = "tc"):
         """scripts/3:98-162."""
         import os
-        activations = self.get_activations_many([rqae], layers=layers, top_k=top_k)[0]
+        activations = self.get_activations_many([rqae], layers=layers, top_k=top_k, precision=precision)[0]
         if index is not None:
             rqae.activations = activations
             os.makedirs(self.feature_folder, exist_ok=True)
@@ -367,14 +409,15 @@ SCRIPT3_LAYERS = [2, 4, 6, 8, 12, 16, 24, 32, 48, 64, 128, 256, 512, 1023]   # s
 
 
 def make_feature(rqae, feature_helper: "FeatureHelper", num_tokens: int = 1024, layers: Optional[List[int]] = None,
-                 top_k: int = 100, features_per_launch: int = 64, save: bool = True) -> List["RQAEFeature"]:
+                 top_k: int = 100, features_per_launch: int = 64, save: bool = True,
+                 precision: str = "tc") -> List["RQAEFeature"]:
     """The driver of ``scripts/3_make_rqae_features.py:164-200`` on one GPU: one random occurrence per distinct token
     (``get_unique_token_indices``), the 200 lowest and highest token ids dropped, shuffled, the first ``num_tokens``
     kept (:167-172; two draws from the global generator, as in the reference); each becomes an ``RQAEFeature`` centred
     on that token's codes (:184-188) whose activations are mined over the whole store and saved as
     ``<feature_folder>/{i:06d}.npz`` (:150-158).  Where the reference spawns one container per feature (:189-191),
     ``features_per_launch`` features share one intensity GEMM and one selection launch (64 features x 14 cuts x
-    4.7 M tokens of fp16 intensities = 8.4 GB)."""
+    4.7 M tokens of fp16 intensities = 8.4 GB).  ``precision="exact"`` mines from the reference's own intensity values."""
     import os
     layers = list(SCRIPT3_LAYERS if layers is None else layers)
     picks = feature_helper.get_unique_token_indices()
@@ -383,6 +426,7 @@ def make_feature(rqae, feature_helper: "FeatureHelper", num_tokens: int = 1024, 
     picks = picks[:num_tokens]
     centers = feature_helper.get_token_indices(picks)
     lw = layer_weights_f16(rqae)          # once: from_quantizer would recompute it (num_quantizers host syncs) per feature
+    kw = {} if precision == "tc" else {"precision": precision}   # the default keeps get_activations_many's old call
     features = []
     for i in range(picks.shape[0]):
         f = RQAEFeature(num_quantizers=rqae.num_quantizers, dim=rqae.codebook_dim, center=centers[i].cpu().numpy(), layers=layers)
@@ -390,7 +434,7 @@ def make_feature(rqae, feature_helper: "FeatureHelper", num_tokens: int = 1024, 
         features.append(f)
     for f0 in range(0, len(features), features_per_launch):
         group = features[f0:f0 + features_per_launch]
-        for j, acts in enumerate(feature_helper.get_activations_many(group, layers=layers, top_k=top_k)):
+        for j, acts in enumerate(feature_helper.get_activations_many(group, layers=layers, top_k=top_k, **kw)):
             group[j].activations = acts
             if save:
                 os.makedirs(feature_helper.feature_folder, exist_ok=True)

@@ -124,7 +124,7 @@ class RQAE(nn.Module):
     def _apply(self, fn, *args, **kwargs):
         self._packed = None
         self.__dict__.pop("_tc_weights", None)
-        for k in ("_codebook_sims", "_subfeatures", "_subfeature_sims", "_layer_norms"):
+        for k in ("_codebook_sims", "_subfeatures", "_subfeature_sims", "_layer_norms", "_exact_sims"):
             self.__dict__.pop(k, None)
         return super()._apply(fn, *args, **kwargs)
 
